@@ -17,6 +17,7 @@ With --gpus N the V pairs are block-partitioned over N ranks (configs[2]); total
 `--impl reference` times that CPU path alone (rank 0 only) and prints the same JSON shape.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -57,7 +58,48 @@ def parse_args():
                     help="N GPUs from ONE process through mvr_register_turntable_multi (one host thread per GPU, ncclAllGather inside the "
                          "C ABI); the default for --gpus N > 1 when not launched by torchrun")
     ap.add_argument("--streams", type=int, default=1, help="GPU contexts created up front (the driver grows the pool to one per pair)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 or float64, "
+                         "at most 64 MB; the NN sweep writes a fixed sample of its answers), so that two builds can be compared "
+                         "output for output")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 << 20
+NN_DUMP_SAMPLE = 1 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array.  float32 arrays stay float32; everything else (float64, counts,
+    indices) is written as float64, which holds each of these values exactly."""
+    out = {}
+    for name, x in arrays.items():
+        x = np.asarray(x)
+        out[name] = np.ascontiguousarray(x, dtype=np.float32 if x.dtype == np.float32 else np.float64)
+    total = sum(x.nbytes for x in out.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes, more than %d" % (total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for name, x in out.items():
+        np.save(os.path.join(path, name + ".npy"), x)
+
+
+def registration_outputs(view_poses, records):
+    """What a caller of the turntable registration receives: the absolute pose of every view (V x 4 x 4) and the result of
+    every ring pair (the gathered pair records)."""
+    import mvr_b200.ring as ring
+    rec = np.asarray(records).view(ring.RECORD).reshape(-1)
+    return {"view_poses": np.asarray(view_poses, dtype=np.float32).reshape(-1, 4, 4),
+            "pair_poses": rec["pose"].reshape(-1, 4, 4).transpose(0, 2, 1),
+            "pair_n_corr": rec["n_corr"], "pair_iterations": rec["iterations"], "pair_status": rec["status"],
+            "pair_mse": rec["mse"], "pair_nn_queries": rec["nn_queries"]}
+
+
+def nn_sample(n):
+    """Fixed positions of the NN answers --dump-outputs keeps: at most NN_DUMP_SAMPLE of n, seeded, in ascending order."""
+    if n <= NN_DUMP_SAMPLE:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, NN_DUMP_SAMPLE, replace=False))
 
 
 def workload_config(a, world):
@@ -160,9 +202,13 @@ def run_reference(a):
         cpu_align_pairs(a, views, pairs[:1])
     tq, tt, cores = 0, 0.0, 1
     for _ in range(a.steps):
-        q, dt, cores = cpu_align_pairs(a, views, pairs)
+        last = []
+        q, dt, cores = cpu_align_pairs(a, views, pairs, keep=last)
         tq += q
         tt += dt
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"pair_poses": np.stack([o["final"] for o in last]),
+                                      **{"pair_" + k: [o[k] for o in last] for k in ("n_corr", "iterations", "status", "mse", "nn_queries")}})
     val = tq / tt
     q1, dt1, _ = cpu_align_pairs(a, views, pairs[:1], threads=1, iters=max(1, a.iters // 3))
     sample = "pairs 0..%d of the sequence (%d/%d of a step), %d iterations, per step" % (ns - 1, ns, a.views, a.iters)
@@ -194,6 +240,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", "-i", str(index), "--query-gpu=" + self.FIELDS, "--format=csv,noheader,nounits", "-lms", "100"],
                                       stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)   # a run that fails before stop() must not leave the sampler running
         except OSError:
             self.p = None
 
@@ -358,6 +405,11 @@ def run_native(a):
     q = allsum(q)
     launches = allsum(launches)
     value = q / (ms * 1e-3)
+    if a.dump_outputs and rank == 0:
+        step_poses, allrec = last[1]
+        if world == 1:   # the driver's V x 16 column-major poses
+            step_poses = step_poses.reshape(-1, 4, 4).transpose(0, 2, 1)
+        dump_outputs(a.dump_outputs, registration_outputs(step_poses, allrec))
 
     # ---- end-to-end leg (host buffers through the C ABI) ----
     e2e = None
@@ -559,6 +611,8 @@ def run_single_process(a):
     w1 = time.time()
     launches = mvr_b200.kernel_launch_count() - l0
     clocks = sampler.stop(w0, w1)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, registration_outputs(last[0], last[2]))
     e2e = None
     if not a.no_e2e:
         for _ in range(max(1, min(a.warmup, 2))):
@@ -593,7 +647,8 @@ def nn_config(a):
             "l2": "queries + results of the headline step are 384 MB (> 126 MB L2): no flush needed"}
 
 
-def nn_cpu(a, tgt, q, threads):
+def nn_cpu(a, tgt, q, threads, keep=None):
+    """keep (list): receives the answers (indices, d2) of the last repetition."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import oracle
     oracle.build()
@@ -602,9 +657,11 @@ def nn_cpu(a, tgt, q, threads):
     best = None
     for _ in range(max(a.cpu_reps, 1)):
         t0 = time.perf_counter()
-        tree.query(q)
+        ans = tree.query(q)
         dt = time.perf_counter() - t0
         best = dt if best is None else min(best, dt)
+    if keep is not None:
+        keep.extend(ans)
     return len(q) / best, best, oracle.num_threads()
 
 
@@ -614,7 +671,11 @@ def run_nn_reference(a):
     import mvr_b200.synth as synth
     ns = min(a.nn_queries, 2_000_000)
     tgt, q = synth.nn_sweep_case(a.nn_target, ns, order="random")
-    val, sec, cores = nn_cpu(a, tgt, q, host_threads())
+    last = []
+    val, sec, cores = nn_cpu(a, tgt, q, host_threads(), keep=last)
+    if a.dump_outputs:
+        sel = nn_sample(ns)
+        dump_outputs(a.dump_outputs, {"query_index": sel, "nn_index": last[0][sel], "nn_d2": last[1][sel]})
     v1, s1, _ = nn_cpu(a, tgt, q[:200_000], 1)
     print(json.dumps({
         "impl": "reference", "metric": NN_METRIC, "value": val, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup,
@@ -693,6 +754,10 @@ def run_nn_sweep(a):
     launches = mvr_b200.kernel_launch_count() - l0
     clocks = sampler.stop(w0, w1) if sampler else None
     value = a.nn_queries * a.steps / (ms * 1e-3)
+    if a.dump_outputs and rank == 0:   # rank 0's share of the queries (under torchrun), sampled
+        sel = nn_sample(nq)
+        ts = torch.from_numpy(sel).to(dev)
+        dump_outputs(a.dump_outputs, {"query_index": sel, "nn_index": di[ts].cpu().numpy(), "nn_d2": dd[ts].cpu().numpy()})
     e2e = None
     if not a.no_e2e:
         timed(1, True)

@@ -35,14 +35,21 @@ def test_built_for_sm_100a_only():
     assert archs == {"sm_100a"}, archs
 
 
+def _without_a_device(code):
+    """Runs `code` in a child process that sees no CUDA device (CUDA_VISIBLE_DEVICES empty), whether or not the machine has one."""
+    r = subprocess.run([sys.executable, "-c", "import sys\nsys.path.insert(0, %r)\n%s" % (ROOT, code)],
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True, timeout=120)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+
+
 def test_no_cpu_fallback_without_a_device(mvr):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a CUDA device is present")
-    with pytest.raises(mvr.MvrError):
-        mvr.Context(0)
-    with pytest.raises(mvr.MvrError):
-        mvr.Registrator(0, 2)
+    _without_a_device(
+        "import pytest\n"
+        "import mvr_b200 as mvr\n"
+        "with pytest.raises(mvr.MvrError):\n"
+        "    mvr.Context(0)\n"
+        "with pytest.raises(mvr.MvrError):\n"
+        "    mvr.Registrator(0, 2)\n")
 
 
 def test_product_never_touches_the_oracle():
@@ -391,12 +398,11 @@ def test_pair_record_layout_matches_the_header(mvr):
 
 
 def test_multi_create_without_gpu_fails_loudly(mvr):
-    import ctypes
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("needs a box without a GPU")
-    h = ctypes.c_void_p()
-    assert mvr.lib().mvr_multi_create(None, 2, ctypes.byref(h)) == mvr.ERR_CUDA and not h.value
+    _without_a_device(
+        "import ctypes\n"
+        "import mvr_b200 as mvr\n"
+        "h = ctypes.c_void_p()\n"
+        "assert mvr.lib().mvr_multi_create(None, 2, ctypes.byref(h)) == mvr.ERR_CUDA and not h.value\n")
 
 
 def _lum_ring(orc, synth, V=6, n=6000):
