@@ -77,6 +77,7 @@ class TurntableParams(C.Structure):
         ("pair_begin", C.c_int),
         ("pair_end", C.c_int),
         ("want_fitness", C.c_int),
+        ("normal_k", C.c_int),
     ]
 
 
@@ -201,6 +202,7 @@ def lib():
     L.mvr_fitness_score.argtypes = [vp, C.c_double, C.POINTER(C.c_double)]
     L.mvr_denoise.argtypes = [vp, vp, C.c_size_t, C.c_size_t, C.c_int, C.c_double, ip, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
     L.mvr_estimate_normals.argtypes = [vp, C.c_int, C.c_int, fp, fp, ip]
+    L.mvr_estimate_normals_batch.argtypes = [C.POINTER(vp), C.c_int, C.c_int, fp, C.POINTER(fp), ip]
     dp = C.POINTER(C.c_double)
     L.mvr_apply_pose.argtypes = [vp, vp, C.c_size_t, C.c_size_t, dp, fp]
     L.mvr_apply_pose_device.argtypes = [vp, vp, C.c_size_t, C.c_size_t, dp, vp]
@@ -317,6 +319,7 @@ class Context:
 
     def __init__(self, device=0, _borrowed=None):
         self._keep = {}
+        self._tgt_n = None   # points of the target set through this object (sizes the host copies of estimate_normals_batch)
         self._owned = _borrowed is None
         if _borrowed is not None:
             self._h = C.c_void_p(_borrowed)
@@ -388,6 +391,7 @@ class Context:
     def set_target(self, pts):
         pts = _pts(pts)
         self._ck(lib().mvr_set_target(self._h, pts.ctypes.data, len(pts)))
+        self._tgt_n = len(pts)
 
     def set_source(self, pts):
         pts = _pts(pts)
@@ -396,6 +400,7 @@ class Context:
     def set_target_device(self, ptr, n, keepalive=None):
         self._keep["tgt"] = keepalive
         self._ck(lib().mvr_set_target_device(self._h, C.c_void_p(int(ptr)), int(n)))
+        self._tgt_n = int(n)
 
     def set_source_device(self, ptr, n, keepalive=None):
         self._keep["src"] = keepalive
@@ -650,6 +655,9 @@ def set_clouds_device(contexts, which, ptrs, counts, keepalive=None):
     rc = lib().mvr_set_clouds_device(hs, _ip(w), pp, cc, n)
     if rc != OK:
         raise MvrError(rc, contexts[0].last_error() if n else "")
+    for k, c in enumerate(contexts):
+        if int(w[k]) == TARGET:
+            c._tgt_n = int(counts[k])
 
 
 def icp_align_batch(contexts, params, guesses=None):
@@ -669,6 +677,28 @@ def icp_align_batch(contexts, params, guesses=None):
     return [dict(status=int(st[k]), final=pose_to_numpy(fin[k]), iterations=reps[k].iterations, converged=bool(reps[k].converged),
                  reason=reps[k].reason, n_corr=reps[k].n_correspondences, mse=reps[k].mse, gpu_ms=reps[k].gpu_ms,
                  nn_queries=int(reps[k].nn_queries)) for k in range(n)]
+
+
+def estimate_normals_batch(contexts, k, viewpoints=None, want=False):
+    """mvr_estimate_normals_batch: kNN(k) PCA normals of every context's TARGET (the same bits as Context.estimate_normals),
+    kept on the device for point-to-plane ICP.  viewpoints: len(contexts) x 3 (None: each target's origin).  Returns a list
+    with, per context, its n x 4 float32 {nx, ny, nz, curvature} when want is true, else None.  Raises on a failed status."""
+    n = len(contexts)
+    hs = (C.c_void_p * max(n, 1))(*[c._h for c in contexts])
+    vp = None if viewpoints is None else np.ascontiguousarray(np.asarray(viewpoints, dtype=np.float32).reshape(n, 3))
+    outs = [None] * n
+    ptrs = None
+    if want:
+        outs = [np.empty((c._tgt_n, 4), dtype=np.float32) if c._tgt_n is not None else None for c in contexts]
+        ptrs = (C.POINTER(C.c_float) * max(n, 1))(*[_fp(o) if o is not None else C.POINTER(C.c_float)() for o in outs])
+    st = np.zeros(max(n, 1), dtype=np.int32)
+    rc = lib().mvr_estimate_normals_batch(hs, n, int(k), _fp(vp) if vp is not None else None, ptrs, _ip(st))
+    if rc != OK:
+        raise MvrError(rc, contexts[0].last_error() if n else lib().mvr_status_string(rc).decode())
+    for i in range(n):
+        if st[i] != OK:
+            raise MvrError(int(st[i]), contexts[i].last_error() or lib().mvr_status_string(int(st[i])).decode())
+    return outs
 
 
 def pair_moments_transform(m, pose, new_origin=None):

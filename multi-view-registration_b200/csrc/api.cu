@@ -551,6 +551,24 @@ void parallel_for(int n, F fn) {
   for (std::thread& t : th) t.join();
 }
 
+// Grid of the index mvr_estimate_normals builds over cloud c: the cell edge is ~1.25 x the expected distance of the k-th
+// neighbour on a surface of the cloud's density, so the 27 cells around a point hold its k neighbours and prove it (the k-th
+// distance is below one cell) for nearly every point.
+PairGrid normals_grid(const mvr_ctx* ctx, const Cloud& c, int k, uint32_t* cells) {
+  const double e = ctx->cell_edge_opt > 0 ? ctx->cell_edge_opt : density_cell_edge(c.lo, c.hi, c.n - c.n_bad, std::max(2.0, k / 3.0));
+  return make_pair_grid(c.lo, c.hi, e, cells);
+}
+
+// The normals of the n points indexed by ix: viewpoint NULL = the origin.
+NormalsJob normals_job(const PairIndex& ix, int n, const float* viewpoint, float4* out, int32_t* nbr) {
+  NormalsJob j{};
+  j.sorted = ix.sorted.as<float4>(); j.start = ix.start.as<uint32_t>(); j.g = ix.g;
+  j.n = n; j.n_valid = ix.n_valid;
+  j.viewpoint = viewpoint ? make_float3(viewpoint[0], viewpoint[1], viewpoint[2]) : make_float3(0.f, 0.f, 0.f);
+  j.out = out; j.nbr = nbr;
+  return j;
+}
+
 
 }  // namespace
 
@@ -1625,22 +1643,20 @@ int mvr_estimate_normals(mvr_ctx* ctx, int which, int k, const float viewpoint[3
   if (c.gen == 0) return fail(ctx, MVR_ERR_NO_INPUT, "cloud not set");
   const int n = c.n;
   if (n == 0) return MVR_OK;
-  // the cell edge is ~1.25 x the expected distance of the k-th neighbour on a surface of the cloud's density: the 27 cells around
-  // a point then hold its k neighbours and prove it (the k-th distance is below one cell) for nearly every point
-  const double e = ctx->cell_edge_opt > 0 ? ctx->cell_edge_opt : density_cell_edge(c.lo, c.hi, n - c.n_bad, std::max(2.0, k / 3.0));
   uint32_t cells = 0;
-  const PairGrid g = make_pair_grid(c.lo, c.hi, e, &cells);
+  const PairGrid g = normals_grid(ctx, c, k, &cells);
   PairIndex& ix = ctx->nq;
   int rc = build_pair_index(ctx, ix, c.pts, n, c.n_bad, nullptr, g, cells, false, false);
   if (rc) return rc;
-  float3 vp = viewpoint ? make_float3(viewpoint[0], viewpoint[1], viewpoint[2]) : make_float3(0.f, 0.f, 0.f);
   DevBuf& nb = which == MVR_CLOUD_TARGET ? ctx->normals : ctx->qtmp;
   CK(nb.ensure((size_t)n * sizeof(float4)));
   int32_t* dn = nullptr;
   if (neighbours) { CK(ctx->itmp.ensure((size_t)n * k * sizeof(int32_t))); dn = ctx->itmp.as<int32_t>(); }
+  NormalsBatch batch;
+  batch.j[0] = normals_job(ix, n, viewpoint, nb.as<float4>(), dn);
   {
     ProfScope ps(ctx, MVR_K_NORMALS, 32.0 * n, n);
-    CK(launch_normals(ix.sorted.as<float4>(), ix.start.as<uint32_t>(), g, n, ix.n_valid, k, vp, nb.as<float4>(), dn, ctx->stream));
+    CK(launch_normals(batch, 1, k, ctx->stream));
   }
   ix.valid = false;
   CK(cudaMemcpyAsync(out, nb.p, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1648,6 +1664,79 @@ int mvr_estimate_normals(mvr_ctx* ctx, int which, int k, const float viewpoint[3
   CK(cudaStreamSynchronize(ctx->stream));
   if (which == MVR_CLOUD_TARGET) ctx->has_normals = true;
   return MVR_OK;
+}
+
+// The target normals of many contexts: every index is planned on the host, then the builds (four launches per BUILD_MAX_JOBS
+// clouds, run_pair_builds) and the normals (one launch per BUILD_MAX_JOBS clouds) go to the LEAD's stream.  That stream first
+// waits for the work already queued on every context's stream (their targets and buffers), and every context's stream then
+// waits for the normals, so whatever a context does next -- on its own stream or on the stream of the align group it joins --
+// runs after them.  The grids and the kernel are those of mvr_estimate_normals: the same bits, whatever the batch.
+int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const float* viewpoints, float* const* out_nxyzc, int* statuses) {
+  if (count < 0 || (count && (!ctxs || !statuses))) return MVR_ERR_BAD_ARG;
+  if (count == 0) return MVR_OK;
+  for (int a = 0; a < count; ++a) {
+    if (!ctxs[a]) return MVR_ERR_BAD_ARG;
+    for (int b = 0; b < a; ++b) if (ctxs[b] == ctxs[a]) return fail(ctxs[0], MVR_ERR_BAD_ARG, "a context appears twice in the batch");
+    if (ctxs[a]->device != ctxs[0]->device) return fail(ctxs[0], MVR_ERR_BAD_ARG, "the contexts of a batch must share a device");
+  }
+  mvr_ctx* ctx = ctxs[0];   // the lead: CK() reports into it, its stream runs the batch, its profile records the launches
+  if (k < 3 || k > 32) return fail(ctx, MVR_ERR_BAD_ARG, "k must be in 3..32");
+  cudaSetDevice(ctx->device);
+  const cudaStream_t S = ctx->stream;
+  cudaEvent_t ev = get_event(ctx);
+  if (!ev) return fail(ctx, MVR_ERR_CUDA, "cudaEventCreate failed");
+  struct Todo { mvr_ctx* m; int slot; NormalsJob job; };
+  std::vector<Todo> todo;
+  std::vector<BuildJob> builds;
+  int rc = MVR_OK;
+  for (int a = 0; a < count && rc == MVR_OK; ++a) {
+    mvr_ctx* m = ctxs[a];
+    if (m != ctx && m->stream != S) {
+      if (cudaEventRecord(ev, m->stream) != cudaSuccess || cudaStreamWaitEvent(S, ev, 0) != cudaSuccess) rc = fail(ctx, MVR_ERR_CUDA, "stream ordering failed");
+    }
+    if (rc) break;
+    Cloud& t = m->tgt;
+    if (t.gen == 0) { statuses[a] = fail(m, MVR_ERR_NO_INPUT, "target not set"); continue; }
+    statuses[a] = MVR_OK;
+    if (t.n == 0) continue;
+    uint32_t cells = 0;
+    const PairGrid g = normals_grid(m, t, k, &cells);
+    BuildJob bj;
+    m->nq.valid = false;
+    if ((rc = plan_pair_index(m, m->nq, 1, t.pts, t.n, t.n_bad, nullptr, g, cells, false, S, &bj))) { ctx->err = m->err; break; }
+    if (m->normals.ensure((size_t)t.n * sizeof(float4)) != cudaSuccess) { rc = fail(ctx, MVR_ERR_CUDA, "normals buffer allocation failed"); break; }
+    builds.push_back(bj);
+    todo.push_back(Todo{m, a, normals_job(m->nq, t.n, viewpoints ? viewpoints + 3 * a : nullptr, m->normals.as<float4>(), nullptr)});
+  }
+  if (rc == MVR_OK) rc = run_pair_builds(ctx, builds.data(), (int)builds.size(), S);
+  for (size_t t0 = 0; rc == MVR_OK && t0 < todo.size(); t0 += BUILD_MAX_JOBS) {
+    const int c = (int)std::min(todo.size() - t0, (size_t)BUILD_MAX_JOBS);
+    NormalsBatch batch;
+    double pts = 0;
+    for (int a = 0; a < c; ++a) { batch.j[a] = todo[t0 + a].job; pts += todo[t0 + a].job.n; }
+    ProfScope ps(ctx, MVR_K_NORMALS, 32.0 * pts, pts, 1, S);
+    const cudaError_t e = launch_normals(batch, c, k, S);
+    if (e != cudaSuccess) rc = fail(ctx, MVR_ERR_CUDA, (std::string("launch_normals: ") + cudaGetErrorString(e)).c_str());
+  }
+  bool copies = false;
+  for (size_t a = 0; rc == MVR_OK && a < todo.size(); ++a) {
+    mvr_ctx* m = todo[a].m;
+    m->nq.valid = false;
+    m->has_normals = true;
+    float* out = out_nxyzc ? out_nxyzc[todo[a].slot] : nullptr;
+    if (!out) continue;
+    if (cudaMemcpyAsync(out, m->normals.p, (size_t)m->tgt.n * sizeof(float4), cudaMemcpyDeviceToHost, S) != cudaSuccess) rc = fail(ctx, MVR_ERR_CUDA, "normals copy failed");
+    copies = true;
+  }
+  // every context's later work waits for the normals (also after a failure: nothing queued above may overlap it)
+  if (cudaEventRecord(ev, S) == cudaSuccess) {
+    for (int a = 0; a < count; ++a) if (ctxs[a]->stream != S) cudaStreamWaitEvent(ctxs[a]->stream, ev, 0);
+  } else if (rc == MVR_OK) {
+    rc = fail(ctx, MVR_ERR_CUDA, "stream ordering failed");
+  }
+  ctx->ev_pool.push_back(ev);
+  if (rc == MVR_OK && copies) CK(cudaStreamSynchronize(S));
+  return rc;
 }
 
 }  // extern "C"

@@ -245,9 +245,20 @@ cudaError_t launch_denoise_keys(const uint32_t* count, int n, uint32_t segment_t
                                 uint32_t* n_noise, cudaStream_t s);
 
 // ---- normals.cu ----------------------------------------------------------------------------
-// sorted / start / g: a row-major index of the cloud (pair_index.cu; the order inside a cell does not matter), n points of which
-// the first n_valid sorted positions are finite.  out_nxyzc / out_nbr are indexed by ORIGINAL point index.
-cudaError_t launch_normals(const float4* sorted, const uint32_t* start, PairGrid g, int n, int n_valid, int k, float3 viewpoint, float4* out_nxyzc,
-                           int32_t* out_nbr, cudaStream_t s);
+// One cloud: sorted / start / g: a row-major index of it (pair_index.cu; the order inside a cell does not matter), n points of
+// which the first n_valid sorted positions are finite.  out (n x {nx, ny, nz, curvature}) and nbr (nullable, n x k) are indexed
+// by ORIGINAL point index.
+struct NormalsJob {
+  const float4* sorted;
+  const uint32_t* start;
+  PairGrid g;
+  int n, n_valid;
+  float3 viewpoint;
+  float4* out;
+  int32_t* nbr;
+};
+struct NormalsBatch { NormalsJob j[BUILD_MAX_JOBS]; };
+// kNN(k) PCA normals of `count` (<= BUILD_MAX_JOBS) clouds in one launch, all with the same k.
+cudaError_t launch_normals(const NormalsBatch& batch, int count, int k, cudaStream_t s);
 
 }  // namespace mvr

@@ -11,6 +11,8 @@
 // thread, every insertion a chain of local loads and stores: 4.9 ms for 2M points).  The list is sorted once at the end
 // (neighbours are reported in ascending (d2, index)), then two-pass covariance in double, Jacobi eigen-solve,
 // normal = eigenvector of the smallest eigenvalue flipped towards the viewpoint, curvature = l0 / (l0 + l1 + l2).
+#include <algorithm>
+
 #include "launch.h"
 #include "pair_search.cuh"
 #include "small_solve.h"
@@ -47,14 +49,25 @@ struct KnnList {
   __device__ __forceinline__ float worst_d() const { return n < k ? MVR_INF : wd; }
 };
 
+// One launch serves every cloud of a NormalsBatch: blockIdx.y selects the job, blockIdx.x < ceil(n / KN_THREADS) of that job
+// does its work (the jobs travel by value in the kernel's parameter space, as the builds of pair_index.cu do).  k <= 16 asks
+// for eight blocks per SM: the single-cloud kernel this replaced got 64 registers (eight blocks) unasked; without the bound the
+// job-indexed parameters take it to 72 (seven blocks).
 template <int KMAX>
-__global__ void __launch_bounds__(KN_THREADS) k_normals(const float4* __restrict__ sorted, const uint32_t* __restrict__ start, PairGrid g, int n, int n_valid,
-                                                        int k, float3 vp, float4* __restrict__ out, int32_t* __restrict__ nbr) {
+__global__ void __launch_bounds__(KN_THREADS, KMAX <= 16 ? 8 : 0) k_normals(const __grid_constant__ NormalsBatch b, int k) {
   __shared__ float s_d[KMAX * KN_THREADS];     // k <= KMAX: 24 KB per block for k <= 16 (nine blocks per SM), 48 KB above
   __shared__ int s_id[KMAX * KN_THREADS];
   __shared__ int s_pos[KMAX * KN_THREADS];
+  const NormalsJob& j = b.j[blockIdx.y];
   const int sp = blockIdx.x * KN_THREADS + threadIdx.x;
-  if (sp >= n) return;
+  if (sp >= j.n) return;
+  const float4* __restrict__ sorted = j.sorted;
+  const uint32_t* __restrict__ start = j.start;
+  const PairGrid& g = j.g;
+  const int n_valid = j.n_valid;
+  float4* __restrict__ out = j.out;
+  int32_t* __restrict__ nbr = j.nbr;
+  const float3 vp = j.viewpoint;
   const float4 q = __ldg(sorted + sp);
   const int self = __float_as_int(q.w);
   if (sp >= n_valid) {  // non-finite point
@@ -138,13 +151,15 @@ __global__ void __launch_bounds__(KN_THREADS) k_normals(const float4* __restrict
   out[self] = make_float4((float)nx, (float)ny, (float)nz, (float)(tr > 0 ? fabs(w[0] / tr) : 0.0));
 }
 
-cudaError_t launch_normals(const float4* sorted, const uint32_t* start, PairGrid g, int n, int n_valid, int k, float3 viewpoint, float4* out_nxyzc,
-                           int32_t* out_nbr, cudaStream_t s) {
-  if (n <= 0) return cudaSuccess;
-  if (k < 1 || k > KNN_MAX) return cudaErrorInvalidValue;
-  const int blocks = (n + KN_THREADS - 1) / KN_THREADS;
-  if (k <= 16) k_normals<16><<<blocks, KN_THREADS, 0, s>>>(sorted, start, g, n, n_valid, k, viewpoint, out_nxyzc, out_nbr);
-  else k_normals<KNN_MAX><<<blocks, KN_THREADS, 0, s>>>(sorted, start, g, n, n_valid, k, viewpoint, out_nxyzc, out_nbr);
+cudaError_t launch_normals(const NormalsBatch& batch, int count, int k, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  if (count > BUILD_MAX_JOBS || k < 1 || k > KNN_MAX) return cudaErrorInvalidValue;
+  int max_n = 0;
+  for (int a = 0; a < count; ++a) max_n = std::max(max_n, batch.j[a].n);
+  if (max_n <= 0) return cudaSuccess;
+  const dim3 grid((unsigned)((max_n + KN_THREADS - 1) / KN_THREADS), (unsigned)count);
+  if (k <= 16) k_normals<16><<<grid, KN_THREADS, 0, s>>>(batch, k);
+  else k_normals<KNN_MAX><<<grid, KN_THREADS, 0, s>>>(batch, k);
   count_launch();
   return cudaGetLastError();
 }

@@ -48,6 +48,7 @@ void mvr_turntable_params_default(mvr_turntable_params* p) {
   p->mode = MVR_REGISTER_RING_PAIRS;
   p->loop_closure = 1;
   p->lum_iterations = 16;                     // mvr/src/registrator.cpp:623
+  p->normal_k = 16;
 }
 
 void mvr_turntable_rotation(const double pivot[3], const double axis[3], double angle, double* out16) {

@@ -383,6 +383,8 @@ int Registrator::automaticRegistration(std::vector<View>& views, int max_iterati
 
 int Registrator::multiViewRegister(std::vector<View>& views, const mvr_turntable_params& prm, std::vector<mvr_pair_report>& reports) {
   if (!ok()) return fail(MVR_ERR_CUDA, "no GPU context");
+  const int normal_k = prm.normal_k == 0 ? 16 : prm.normal_k;   // 0: a zero-filled struct gets the default
+  if (normal_k < 3 || normal_k > 32) return fail(MVR_ERR_BAD_ARG, "normal_k must be in 3..32 (0: 16)");
   const int V = (int)views.size();
   reports.assign((size_t)std::max(V, 0), mvr_pair_report{});
   if (V < 2) return MVR_OK;
@@ -442,6 +444,13 @@ int Registrator::multiViewRegister(std::vector<View>& views, const mvr_turntable
     else rc = mvr_set_source_device(ctx_[(size_t)k], dview[(size_t)sv], views[(size_t)sv].size);
     if (rc) return fail(rc, mvr_last_error(ctx_[(size_t)k]));
   }
+  // point-to-plane: the target normals of every pair in one batch, each towards the origin of its view's own sensor frame (PCL's
+  // default viewpoint); a pure function of the view, so pair poses do not depend on how the ring is sharded.  The repeats
+  // reuse them; a source (shared or not) needs none.
+  if (prm.icp.estimator == MVR_POINT_TO_PLANE) {
+    if ((rc = mvr_estimate_normals_batch(cs.data(), P, normal_k, nullptr, nullptr, st.data()))) return fail(rc, mvr_last_error(cs[0]));
+    for (int k = 0; k < P; ++k) if (st[(size_t)k]) return fail(st[(size_t)k], mvr_last_error(cs[(size_t)k]));
+  }
   const double t_share = now();
   const int repeats = std::max(prm.repeat_times, 1);
   for (int r = 0; r < repeats; ++r) {
@@ -473,7 +482,7 @@ int Registrator::multiViewRegister(std::vector<View>& views, const mvr_turntable
     fill_report(reports[(size_t)p], (p + 1) % V, p, a, iterations[(size_t)k], queries[(size_t)k], ms[(size_t)k], a.final_transformation);
   }
   const double t_align = now();
-  if (timing) std::fprintf(stderr, "[timing] upload+set_target %.3f ms, share %.3f ms, align_batch %.3f ms\n", t_set - t_begin, t_share - t_set, t_align - t_share);
+  if (timing) std::fprintf(stderr, "[timing] upload+set_target %.3f ms, share+normals %.3f ms, align_batch %.3f ms\n", t_set - t_begin, t_share - t_set, t_align - t_share);
   if (p0 == 0 && p1 == V) {
     std::vector<Matrix4d> rel((size_t)V), abs_pose;
     std::vector<double> w((size_t)V);
