@@ -41,7 +41,10 @@ typedef enum {
 } mvr_status;
 
 typedef enum { MVR_CLOUD_TARGET = 0, MVR_CLOUD_SOURCE = 1 } mvr_cloud;
-typedef enum { MVR_POINT_TO_POINT = 0, MVR_POINT_TO_PLANE = 1 } mvr_estimator;
+/* SYMMETRIC: pcl::IterativeClosestPointWithNormals with setUseSymmetricObjective(true), i.e.
+ * TransformationEstimationSymmetricPointToPlaneLLS (PCL >= 1.11) with enforce_same_direction_normals: needs target AND source
+ * normals; the source normals move with the source.  (Other values mean point-to-point.) */
+typedef enum { MVR_POINT_TO_POINT = 0, MVR_POINT_TO_PLANE = 1, MVR_SYMMETRIC = 2 } mvr_estimator;
 typedef enum {
   MVR_REASON_NONE = 0,
   MVR_REASON_ITERATIONS = 1,
@@ -59,7 +62,8 @@ typedef struct {
   double transformation_epsilon;       /* setTransformationEpsilon      (PCL default 0)             */
   double euclidean_fitness_epsilon;    /* setEuclideanFitnessEpsilon    (PCL default -DBL_MAX)      */
   int use_reciprocal_correspondences;  /* setUseReciprocalCorrespondences (reference: true)         */
-  int estimator;                       /* mvr_estimator; the reference only uses point-to-point     */
+  int estimator;                       /* mvr_estimator; the reference only uses point-to-point (point-to-plane needs
+                                          target normals, symmetric needs target and source normals) */
   int fixed_iterations;                /* 1: run exactly max_iterations (bench mode, criteria 2-4 off) */
   int min_correspondences;             /* PCL min_number_correspondences_ = 3                       */
 } mvr_icp_params;
@@ -158,8 +162,16 @@ int mvr_set_clouds_device(mvr_ctx* const* ctxs, const int* which, const float* c
  * nothing is copied or recomputed).  The points must stay alive and unchanged while `dst` uses them -- a view of a
  * turntable ring is the target of one pair and the source of the next. */
 int mvr_cloud_share(mvr_ctx* dst, int which_dst /* mvr_cloud */, mvr_ctx* src, int which_src);
-/* Optional per-target-point normals (n x {nx,ny,nz,curvature}) for point-to-plane ICP. */
+/* Optional per-target-point normals (n x {nx,ny,nz,curvature}) for point-to-plane ICP.  A new target drops them. */
 int mvr_set_target_normals(mvr_ctx* ctx, const float* nxyzc, size_t n);
+/* The same for the source (symmetric ICP): n must equal the source size.  A new source drops them; during an align they turn
+ * with the source (the guess's rotation at its start, each increment's rotation after), on a copy -- these stay as given. */
+int mvr_set_source_normals(mvr_ctx* ctx, const float* nxyzc, size_t n);
+/* Give `dst` the normals another context of the same device holds for its target or source (same device pointer, nothing
+ * copied), like mvr_cloud_share: `src` must keep them alive and unchanged while `dst` uses them.  The two clouds must have
+ * the same number of points (else MVR_ERR_BAD_ARG); MVR_ERR_NO_INPUT if `src` holds no such normals.  A ring view is the
+ * target of one pair and the source of the next: its normals are estimated once. */
+int mvr_normals_share(mvr_ctx* dst, int which_dst /* mvr_cloud */, mvr_ctx* src, int which_src);
 
 /* -- spatial index (replaces pcl::KdTreeFLANN::setInputCloud inside icp.align) ------------------- */
 /* Build the Morton-sorted uniform grid over a cloud with an explicit grid; exported for parity tests. */
@@ -229,7 +241,8 @@ int mvr_pair_moments_compute_batch(mvr_ctx* const* ctxs, int count, double max_d
 
 /* -- extensions named by the north star (no reference call site) -------------------------------- */
 /* pcl::NormalEstimation semantics: kNN(k) PCA normals of a cloud, flipped towards viewpoint.
- * out: n x {nx, ny, nz, curvature}.  neighbours (nullable): n x k int32, ascending (d2, index). */
+ * out: n x {nx, ny, nz, curvature}.  neighbours (nullable): n x k int32, ascending (d2, index).  The result is also kept on the
+ * device as the cloud's normals (target: point-to-plane and symmetric ICP; source: symmetric ICP). */
 int mvr_estimate_normals(mvr_ctx* ctx, int which, int k, const float viewpoint[3], float* out_nxyzc,
                          int32_t* neighbours);
 /* kNN(k) PCA normals of the TARGET cloud of `count` contexts of one device, as mvr_estimate_normals computes them (same
@@ -267,8 +280,8 @@ typedef struct {
 typedef enum {
   MVR_REGISTER_RING_PAIRS = 0,  /* independent neighbour pairs (v+1 -> v, closing pair 0 -> V-1), then loop closure:
                                    the shardable form (ring edges of registrationLUM, mvr/src/registrator.cpp:640-651).
-                                   The only mode that honours icp.estimator (point-to-plane: see normal_k); the others build
-                                   their own point-to-point settings, as the reference does */
+                                   The only mode that honours icp.estimator (point-to-plane and symmetric: see normal_k); the
+                                   others build their own point-to-point settings, as the reference does */
   MVR_REGISTER_ACCUMULATE = 1,  /* automaticRegistration: views 1..V-1 in order, each aligned repeat_times against
                                    the growing model, then refineAxis (mvr/src/registrator.cpp:746-842, 877-990) */
   MVR_REGISTER_ICP = 2,         /* registrationICP: views in the order 1, V-1, 2, V-2, .. against the growing model,
@@ -288,9 +301,11 @@ typedef struct {
   int lum_iterations;      /* relaxation sweeps (reference lum.setMaxIterations(16)) */
   int pair_begin, pair_end;/* ring mode: compute only pairs [begin, end) (multi-GPU sharding); end <= 0 = all V */
   int want_fitness;        /* also run getFitnessScore() after the last align of each pair/view */
-  int normal_k;            /* ring mode with icp.estimator = MVR_POINT_TO_PLANE: neighbours of the target normals, 3..32
-                              (0 = the default, 16).  Each pair's target normals are estimated on the GPU (all pairs in one
-                              batch, mvr_estimate_normals_batch) in the view's own sensor frame, i.e. towards its origin. */
+  int normal_k;            /* ring mode with icp.estimator = MVR_POINT_TO_PLANE or MVR_SYMMETRIC: neighbours of the normals,
+                              3..32 (0 = the default, 16).  Each pair's target normals are estimated on the GPU (all pairs in
+                              one batch, mvr_estimate_normals_batch) in the view's own sensor frame, i.e. towards its origin.
+                              Symmetric: each pair's source normals are those of the pair that has the same view as its target
+                              (mvr_normals_share); the last source of a pair range is estimated in the same batch. */
 } mvr_turntable_params;
 
 typedef struct {

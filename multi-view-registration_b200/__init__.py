@@ -19,7 +19,7 @@ K_COUNT = 8
 (OK, ERR_BAD_ARG, ERR_TOO_FEW, ERR_CUDA, ERR_NO_INPUT, ERR_NOT_SPD, ERR_ALLOC, ERR_NCCL) = range(8)
 TARGET, SOURCE = 0, 1
 NN_AUTO, NN_WARP, NN_THREAD, NN_CELL, NN_SEEDED = 0, 1, 2, 3, 4
-POINT_TO_POINT, POINT_TO_PLANE = 0, 1
+POINT_TO_POINT, POINT_TO_PLANE, SYMMETRIC = 0, 1, 2
 
 
 class MvrError(RuntimeError):
@@ -189,8 +189,10 @@ def lib():
     L.mvr_ctx_set_nn_options.argtypes = [vp, C.c_double, C.c_double]
     L.mvr_ctx_set_nn_mode.argtypes = [vp, C.c_int]
     L.mvr_ctx_set_gate_mask.argtypes = [vp, C.c_int]
-    for name in ("mvr_set_target", "mvr_set_source", "mvr_set_target_device", "mvr_set_source_device", "mvr_set_target_normals"):
+    for name in ("mvr_set_target", "mvr_set_source", "mvr_set_target_device", "mvr_set_source_device", "mvr_set_target_normals",
+                 "mvr_set_source_normals"):
         getattr(L, name).argtypes = [vp, vp, C.c_size_t]
+    L.mvr_normals_share.argtypes = [vp, C.c_int, vp, C.c_int]
     L.mvr_index_build.argtypes = [vp, C.c_int, C.POINTER(Grid)]
     L.mvr_index_export.argtypes = [vp, C.c_int, C.POINTER(Grid), up, ip, up]
     L.mvr_nn_query.argtypes = [vp, fp, C.c_size_t, ip, fp]
@@ -409,6 +411,16 @@ class Context:
     def set_target_normals(self, nrm):
         nrm = _pts(nrm)
         self._ck(lib().mvr_set_target_normals(self._h, nrm.ctypes.data, len(nrm)))
+
+    def set_source_normals(self, nrm):
+        """n x 4 {nx, ny, nz, curvature} of the source (symmetric ICP); n must equal the source size."""
+        nrm = _pts(nrm)
+        self._ck(lib().mvr_set_source_normals(self._h, nrm.ctypes.data, len(nrm)))
+
+    def normals_share(self, which, other, other_which):
+        """mvr_normals_share: this context's TARGET / SOURCE normals become the device normals `other` holds for its
+        `other_which` cloud (no copy; `other` must keep them unchanged while this context uses them)."""
+        self._ck(lib().mvr_normals_share(self._h, int(which), other._h, int(other_which)))
 
     # -- index ---------------------------------------------------------------------------------
     def index_build(self, which=TARGET, grid=None):

@@ -33,6 +33,9 @@ namespace mvr {
 static std::atomic<unsigned long long> g_launches{0};
 void count_launch(int n) { g_launches.fetch_add((unsigned long long)n, std::memory_order_relaxed); }
 unsigned long long launch_count() { return g_launches.load(std::memory_order_relaxed); }
+// host/registrator.h
+int estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int count, int k, const float* viewpoints, float* const* out_nxyzc,
+                           int* statuses);
 }  // namespace mvr
 
 namespace {
@@ -105,7 +108,13 @@ struct mvr_ctx {
   cudaStream_t stream = nullptr;
   bool own_stream = false;
   Cloud tgt, src;
-  DevBuf normals; bool has_normals = false;
+  // normals {nx, ny, nz, curvature} by original point index: tnrm / snrm point at the context's own buffer (normals / snormals)
+  // or at another context's (mvr_normals_share); null: none.  A new cloud drops its normals.
+  DevBuf normals, snormals;
+  const float4* tnrm = nullptr;
+  const float4* snrm = nullptr;
+  DevBuf nsrc;                   // symmetric aligns: the source normals by sorted position, moved with the source
+  Mat4f guess_m{};               // the guess of the prepared align (turns the source normals at its start)
   DevBuf cur, corr_p, corr_j, corr_d2, rmin, rnn, partials, sums, out_cloud, qtmp, itmp, ftmp, scratch, misc, tiles, state, log;
   PairIndex pt, ps;              // target / source index of the running align
   PairIndex nt, nq;              // target / query index of the dense NN pass (cell_nn.cu)
@@ -635,7 +644,7 @@ int mvr_ctx_destroy(mvr_ctx* ctx) {
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   if (ctx->ev_a) cudaEventDestroy(ctx->ev_a);
   if (ctx->ev_b) cudaEventDestroy(ctx->ev_b);
-  ctx->tgt.release(); ctx->src.release(); ctx->normals.release();
+  ctx->tgt.release(); ctx->src.release(); ctx->normals.release(); ctx->snormals.release(); ctx->nsrc.release();
   ctx->pt.release(); ctx->ps.release(); ctx->nt.release(); ctx->nq.release();
   for (auto& b : ctx->bs) { b.keys.release(); b.vals.release(); b.moved.release(); b.count.release(); b.tiles.release(); }
   ctx->stage_dev.release(); ctx->bbox_dev.release();
@@ -729,25 +738,27 @@ int mvr_ctx_set_batch_group(mvr_ctx* ctx, int pairs) {
 int mvr_set_target(mvr_ctx* ctx, const float* xyzw, size_t n) {
   if (!ctx) return MVR_ERR_BAD_ARG;
   cudaSetDevice(ctx->device);
-  ctx->has_normals = false;
+  ctx->tnrm = nullptr;
   return cloud_set(ctx, ctx->tgt, xyzw, n, false);
 }
 int mvr_set_source(mvr_ctx* ctx, const float* xyzw, size_t n) {
   if (!ctx) return MVR_ERR_BAD_ARG;
   cudaSetDevice(ctx->device);
   ctx->have_out = false;
+  ctx->snrm = nullptr;
   return cloud_set(ctx, ctx->src, xyzw, n, false);
 }
 int mvr_set_target_device(mvr_ctx* ctx, const float* d, size_t n) {
   if (!ctx) return MVR_ERR_BAD_ARG;
   cudaSetDevice(ctx->device);
-  ctx->has_normals = false;
+  ctx->tnrm = nullptr;
   return cloud_set(ctx, ctx->tgt, d, n, true);
 }
 int mvr_set_source_device(mvr_ctx* ctx, const float* d, size_t n) {
   if (!ctx) return MVR_ERR_BAD_ARG;
   cudaSetDevice(ctx->device);
   ctx->have_out = false;
+  ctx->snrm = nullptr;
   return cloud_set(ctx, ctx->src, d, n, true);
 }
 
@@ -777,7 +788,7 @@ int mvr_set_clouds_device(mvr_ctx* const* ctxs, const int* which, const float* c
     for (int k = 0; k < c; ++k) {
       mvr_ctx* m = ctxs[k0 + k];
       Cloud& cl = which[k0 + k] == MVR_CLOUD_TARGET ? m->tgt : m->src;
-      if (which[k0 + k] == MVR_CLOUD_TARGET) m->has_normals = false; else { m->have_out = false; m->out_pending = false; }
+      if (which[k0 + k] == MVR_CLOUD_TARGET) m->tnrm = nullptr; else { m->have_out = false; m->out_pending = false; m->snrm = nullptr; }
       cl.index_valid = false;
       cl.gen++;
       cl.n = (int)n[k0 + k];
@@ -804,18 +815,36 @@ int mvr_cloud_share(mvr_ctx* dst, int which_dst, mvr_ctx* src, int which_src) {
   d.gen++;
   d.pts = s.pts; d.n = s.n; d.n_bad = s.n_bad;
   for (int a = 0; a < 3; ++a) { d.lo[a] = s.lo[a]; d.hi[a] = s.hi[a]; }
-  if (which_dst == MVR_CLOUD_TARGET) dst->has_normals = false; else dst->have_out = false;
+  if (which_dst == MVR_CLOUD_TARGET) dst->tnrm = nullptr; else { dst->have_out = false; dst->snrm = nullptr; }
   return MVR_OK;
 }
 
-int mvr_set_target_normals(mvr_ctx* ctx, const float* nxyzc, size_t n) {
+static int set_normals(mvr_ctx* ctx, int which, const float* nxyzc, size_t n) {
   if (!ctx || !nxyzc) return MVR_ERR_BAD_ARG;
   cudaSetDevice(ctx->device);
-  if ((int)n != ctx->tgt.n) return fail(ctx, MVR_ERR_BAD_ARG, "normals count differs from target size");
-  CK(ctx->normals.ensure(std::max<size_t>(n, 1) * sizeof(float4)));
-  CK(cudaMemcpyAsync(ctx->normals.p, nxyzc, n * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
+  const bool tgt = which == MVR_CLOUD_TARGET;
+  if ((int)n != (tgt ? ctx->tgt.n : ctx->src.n)) return fail(ctx, MVR_ERR_BAD_ARG, tgt ? "normals count differs from target size" : "normals count differs from source size");
+  DevBuf& b = tgt ? ctx->normals : ctx->snormals;
+  CK(b.ensure(std::max<size_t>(n, 1) * sizeof(float4)));
+  CK(cudaMemcpyAsync(b.p, nxyzc, n * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  ctx->has_normals = true;
+  (tgt ? ctx->tnrm : ctx->snrm) = b.as<float4>();
+  return MVR_OK;
+}
+
+int mvr_set_target_normals(mvr_ctx* ctx, const float* nxyzc, size_t n) { return set_normals(ctx, MVR_CLOUD_TARGET, nxyzc, n); }
+int mvr_set_source_normals(mvr_ctx* ctx, const float* nxyzc, size_t n) { return set_normals(ctx, MVR_CLOUD_SOURCE, nxyzc, n); }
+
+int mvr_normals_share(mvr_ctx* dst, int which_dst, mvr_ctx* src, int which_src) {
+  if (!dst || !src || (which_dst != MVR_CLOUD_TARGET && which_dst != MVR_CLOUD_SOURCE) ||
+      (which_src != MVR_CLOUD_TARGET && which_src != MVR_CLOUD_SOURCE)) return MVR_ERR_BAD_ARG;
+  if (dst->device != src->device) return fail(dst, MVR_ERR_BAD_ARG, "contexts on different devices");
+  const float4* p = which_src == MVR_CLOUD_TARGET ? src->tnrm : src->snrm;
+  if (!p) return fail(dst, MVR_ERR_NO_INPUT, which_src == MVR_CLOUD_TARGET ? "the other context holds no target normals" : "the other context holds no source normals");
+  const Cloud& sc = which_src == MVR_CLOUD_TARGET ? src->tgt : src->src;
+  const Cloud& dc = which_dst == MVR_CLOUD_TARGET ? dst->tgt : dst->src;
+  if (sc.n != dc.n) return fail(dst, MVR_ERR_BAD_ARG, "normals count differs from the cloud size");
+  (which_dst == MVR_CLOUD_TARGET ? dst->tnrm : dst->snrm) = p;
   return MVR_OK;
 }
 
@@ -883,6 +912,10 @@ int mvr_nn_query(mvr_ctx* ctx, const float* q, size_t n, int32_t* idx, float* d2
 
 static int align_prepare_batch(mvr_ctx* const* ctxs, int count, const mvr_icp_params* prm, const float* guesses, int est, int* statuses,
                                std::vector<mvr_ctx*>& ok, std::vector<int>& slot);
+// mvr_estimator -> the kernels' estimator (an unknown value means point-to-point)
+static int estimator_code(int estimator) {
+  return estimator == MVR_SYMMETRIC ? EST_SYM : (estimator == MVR_POINT_TO_PLANE ? EST_P2L : EST_P2P);
+}
 static int align_prepare(mvr_ctx* ctx, const mvr_icp_params* prm, const float* guess, int est) {
   int st = MVR_OK;
   std::vector<mvr_ctx*> ok;
@@ -957,14 +990,19 @@ static int align_plan(mvr_ctx* ctx, const mvr_icp_params* prm, const float* gues
   Cloud& s = ctx->src;
   const int n = s.n;
   if (n == 0 || ctx->tgt.n == 0) return fail(ctx, MVR_ERR_NO_INPUT, "empty source or target");
-  if (prm->estimator == MVR_POINT_TO_PLANE && !ctx->has_normals)
+  if (prm->estimator == MVR_POINT_TO_PLANE && !ctx->tnrm)
     return fail(ctx, MVR_ERR_NO_INPUT, "point-to-plane needs target normals (mvr_set_target_normals / mvr_estimate_normals)");
+  if (est == EST_SYM && !ctx->tnrm)
+    return fail(ctx, MVR_ERR_NO_INPUT, "symmetric point-to-plane needs target normals (mvr_set_target_normals / mvr_estimate_normals / mvr_normals_share)");
+  if (est == EST_SYM && !ctx->snrm)
+    return fail(ctx, MVR_ERR_NO_INPUT, "symmetric point-to-plane needs source normals (mvr_set_source_normals / mvr_estimate_normals / mvr_normals_share)");
   if (!(prm->max_correspondence_distance >= 0)) return fail(ctx, MVR_ERR_BAD_ARG, "max_correspondence_distance");
   float G[16];
   if (guess) std::memcpy(G, guess, sizeof(G)); else mat_identity(G);
   const bool reciprocal = prm->use_reciprocal_correspondences != 0;
   const double max_dist = prm->max_correspondence_distance;
-  const bool p2l = est == EST_P2L;
+  const bool p2l = est == EST_P2L || est == EST_SYM;
+  const bool sym = est == EST_SYM;
 
   // ---- per-align indices: target over its own box (reused while the target and the grid stay the same),
   //      source over the box of the guessed source
@@ -999,6 +1037,7 @@ static int align_plan(mvr_ctx* ctx, const mvr_icp_params* prm, const float* gues
     const PairGrid gs = make_pair_grid(lo, hi, pair_cell_edge(ctx, s, max_dist), &cells, MVR_PG_XRATIO);
     Mat4f Gm;
     std::memcpy(Gm.m, G, sizeof(Gm.m));
+    ctx->guess_m = Gm;
     BuildJob job;
     ctx->ps.valid = false;
     if ((rc = plan_pair_index(ctx, ctx->ps, 1, s.pts, n, s.n_bad, &Gm, gs, cells, true, S, &job))) { ctx->ps.valid = false; return rc; }
@@ -1008,6 +1047,7 @@ static int align_plan(mvr_ctx* ctx, const mvr_icp_params* prm, const float* gues
   const PairIndex &pt = ctx->pt, &psx = ctx->ps;
   CK(ctx->corr_p.ensure((size_t)std::max(n, 1) * sizeof(int32_t)));   // seeds and gates are filled by launch_align_init
   if (reciprocal) CK(ctx->rmin.ensure((size_t)std::max(m, 1) * sizeof(uint32_t)));
+  if (sym) CK(ctx->nsrc.ensure((size_t)std::max(n, 1) * sizeof(float4)));   // filled by launch_align_init
   CK(ctx->partials.ensure((size_t)std::max((int)FUSED_MAX_BLOCKS, fused_grid_rev(m)) * REDUCE_MAX_VALS * sizeof(double)));
   CK(ctx->state.ensure(sizeof(IcpState)));
   CK(ctx->log.ensure((size_t)ICP_MAX_LOG * sizeof(IterRec)));
@@ -1041,7 +1081,7 @@ static int align_plan(mvr_ctx* ctx, const mvr_icp_params* prm, const float* gues
   h.max_iter = prm->max_iterations;
   h.fixed = prm->fixed_iterations != 0;
   h.min_corr = prm->min_correspondences > 0 ? prm->min_correspondences : 3;
-  h.p2l = p2l; h.recip = reciprocal; h.n_src = n;
+  h.p2l = sym ? 2 : (p2l ? 1 : 0); h.recip = reciprocal; h.n_src = n;
   if (prm->max_iterations <= 0) { h.done = 1; h.reason = MVR_REASON_ITERATIONS; }
   ctx->iters.clear();
   ctx->log_pending = 0;
@@ -1054,12 +1094,13 @@ static int align_plan(mvr_ctx* ctx, const mvr_icp_params* prm, const float* gues
   fa.corr_p = ctx->corr_p.as<int32_t>(); fa.rmin = reciprocal ? ctx->rmin.as<uint32_t>() : nullptr;
   fa.max2 = max_dist * max_dist; fa.max_d2f = gate_float(max_dist);
   fa.gmask = nullptr; fa.gm_stride = 0;   // set by align_prepare_batch once the target index exists
-  fa.nrm = p2l ? ctx->normals.as<float4>() : nullptr;
+  fa.nrm = p2l ? ctx->tnrm : nullptr;
+  fa.nsrc = sym ? ctx->nsrc.as<float4>() : nullptr;
   fa.partials = ctx->partials.as<double>(); fa.st = d_st; fa.log = d_log; fa.grid = fused_grid(psx.n_valid);
   RevArgs& ra = ctx->ra;
   ra = RevArgs{};
   ra.tgt = fa.tgt; ra.m_valid = pt.n_valid; ra.rmin = fa.rmin; ra.cur = fa.cur; ra.sstart = psx.start.as<uint32_t>(); ra.gs = psx.g;
-  ra.n_valid = psx.n_valid; ra.corr_p = fa.corr_p; ra.nrm = fa.nrm;
+  ra.n_valid = psx.n_valid; ra.corr_p = fa.corr_p; ra.nrm = fa.nrm; ra.nsrc = fa.nsrc;
   ra.rnn = nullptr;
   if (reciprocal && ctx->want_rnn) { CK(ctx->rnn.ensure((size_t)std::max(m, 1) * sizeof(int32_t))); ra.rnn = ctx->rnn.as<int32_t>(); }
   ra.partials = fa.partials; ra.st = d_st; ra.log = d_log; ra.grid = fused_grid_rev(pt.n_valid); ra.per = fused_rev_chunks(pt.n_valid);
@@ -1084,6 +1125,7 @@ static InitJob init_job_of(mvr_ctx* c) {
   InitJob j{};
   j.corr_p = c->corr_p.as<int32_t>(); j.n = std::max(c->src.n, 1); j.m = std::max(c->tgt.n, 1);
   j.rmin = c->fa.rmin; j.st = c->state.as<IcpState>(); j.crowded = c->crowded.as<uint32_t>();
+  if (c->fa.nsrc) { j.nsrc = c->fa.nsrc; j.snrm = c->snrm; j.sorted = c->fa.cur; j.n_valid = c->fa.n_valid; j.M = c->guess_m; }
   return j;
 }
 
@@ -1344,7 +1386,7 @@ static int align_finish_collect(mvr_ctx* ctx, mvr_ctx* lead, float* out_pose, mv
   if (ctx->crowded_seen)
     ctx->err = "warning: a grid cell holds " + std::to_string(ctx->crowded_seen) + " points (duplicates or clamped outliers?): index build and search slow down, sums over it lose their fixed order";
   if (h.status == MVR_ERR_TOO_FEW_CORRESPONDENCES) ctx->err = "not enough correspondences";
-  if (h.status == MVR_ERR_NOT_SPD) ctx->err = "point-to-plane normal equations not positive definite";
+  if (h.status == MVR_ERR_NOT_SPD) ctx->err = h.p2l == 2 ? "symmetric point-to-plane normal equations not positive definite" : "point-to-plane normal equations not positive definite";
   return h.status;
 }
 
@@ -1362,12 +1404,12 @@ static int align_finish(mvr_ctx* ctx, mvr_ctx* lead, float* out_pose, float* out
 static int icp_align_impl(mvr_ctx* ctx, const mvr_icp_params* prm, const float* guess, float* out_pose, float* out_xyzw,
                           mvr_icp_report* report, bool moments) {
   if (!ctx || !prm) return MVR_ERR_BAD_ARG;
-  const bool p2l = prm->estimator == MVR_POINT_TO_PLANE;
-  if (moments && p2l) return fail(ctx, MVR_ERR_BAD_ARG, "pair moments are point-to-point statistics");
-  const int est = p2l ? EST_P2L : (moments ? EST_MOM : EST_P2P);
-  int rc = align_prepare(ctx, prm, guess, est);
+  const int est = estimator_code(prm->estimator);
+  if (moments && est != EST_P2P) return fail(ctx, MVR_ERR_BAD_ARG, "pair moments are point-to-point statistics");
+  const int est_run = moments ? EST_MOM : est;
+  int rc = align_prepare(ctx, prm, guess, est_run);
   if (rc) return rc;
-  if ((rc = align_run(&ctx, 1, prm, est))) return rc;
+  if ((rc = align_run(&ctx, 1, prm, est_run))) return rc;
   return align_finish(ctx, ctx, out_pose, out_xyzw, report);
 }
 
@@ -1385,7 +1427,7 @@ int mvr_icp_align_batch(mvr_ctx* const* ctxs, int count, const mvr_icp_params* p
     for (int j = 0; j < k; ++j) if (ctxs[j] == ctxs[k]) return fail(ctxs[0], MVR_ERR_BAD_ARG, "a context appears twice in the batch");
     if (ctxs[k]->device != ctxs[0]->device) return fail(ctxs[0], MVR_ERR_BAD_ARG, "the contexts of a batch must share a device");
   }
-  const int est = prm->estimator == MVR_POINT_TO_PLANE ? EST_P2L : EST_P2P;
+  const int est = estimator_code(prm->estimator);
   std::vector<mvr_ctx*> ok;
   std::vector<int> slot;
   const bool timing = std::getenv("MVR_DEBUG_TIMING") != nullptr;
@@ -1648,7 +1690,7 @@ int mvr_estimate_normals(mvr_ctx* ctx, int which, int k, const float viewpoint[3
   PairIndex& ix = ctx->nq;
   int rc = build_pair_index(ctx, ix, c.pts, n, c.n_bad, nullptr, g, cells, false, false);
   if (rc) return rc;
-  DevBuf& nb = which == MVR_CLOUD_TARGET ? ctx->normals : ctx->qtmp;
+  DevBuf& nb = which == MVR_CLOUD_TARGET ? ctx->normals : ctx->snormals;
   CK(nb.ensure((size_t)n * sizeof(float4)));
   int32_t* dn = nullptr;
   if (neighbours) { CK(ctx->itmp.ensure((size_t)n * k * sizeof(int32_t))); dn = ctx->itmp.as<int32_t>(); }
@@ -1662,21 +1704,30 @@ int mvr_estimate_normals(mvr_ctx* ctx, int which, int k, const float viewpoint[3
   CK(cudaMemcpyAsync(out, nb.p, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
   if (neighbours) CK(cudaMemcpyAsync(neighbours, dn, (size_t)n * k * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  if (which == MVR_CLOUD_TARGET) ctx->has_normals = true;
+  (which == MVR_CLOUD_TARGET ? ctx->tnrm : ctx->snrm) = nb.as<float4>();   // kept as the cloud's normals
   return MVR_OK;
 }
 
-// The target normals of many contexts: every index is planned on the host, then the builds (four launches per BUILD_MAX_JOBS
+// The normals of many clouds of one device: every index is planned on the host, then the builds (four launches per BUILD_MAX_JOBS
 // clouds, run_pair_builds) and the normals (one launch per BUILD_MAX_JOBS clouds) go to the LEAD's stream.  That stream first
-// waits for the work already queued on every context's stream (their targets and buffers), and every context's stream then
+// waits for the work already queued on every context's stream (their clouds and buffers), and every context's stream then
 // waits for the normals, so whatever a context does next -- on its own stream or on the stream of the align group it joins --
 // runs after them.  The grids and the kernel are those of mvr_estimate_normals: the same bits, whatever the batch.
-int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const float* viewpoints, float* const* out_nxyzc, int* statuses) {
+// which (nullable: all targets): entry a estimates the target (MVR_CLOUD_TARGET) or the source normals of ctxs[a]; a context
+// may appear once per cloud.  A target's index is built in the context's query index (nq), a source's in its dense-pass
+// target index (nt, rebuilt by the next NN pass), so both clouds of one context fit in one batch.
+}  // extern "C"
+
+// Declared in host/registrator.h: the ring driver estimates a shard's last source with its targets.
+int mvr::estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int count, int k, const float* viewpoints, float* const* out_nxyzc,
+                                int* statuses) {
   if (count < 0 || (count && (!ctxs || !statuses))) return MVR_ERR_BAD_ARG;
   if (count == 0) return MVR_OK;
+  auto which_of = [&](int a) { return which ? which[a] : (int)MVR_CLOUD_TARGET; };
   for (int a = 0; a < count; ++a) {
-    if (!ctxs[a]) return MVR_ERR_BAD_ARG;
-    for (int b = 0; b < a; ++b) if (ctxs[b] == ctxs[a]) return fail(ctxs[0], MVR_ERR_BAD_ARG, "a context appears twice in the batch");
+    if (!ctxs[a] || (which_of(a) != MVR_CLOUD_TARGET && which_of(a) != MVR_CLOUD_SOURCE)) return MVR_ERR_BAD_ARG;
+    for (int b = 0; b < a; ++b)
+      if (ctxs[b] == ctxs[a] && which_of(b) == which_of(a)) return fail(ctxs[0], MVR_ERR_BAD_ARG, "a context appears twice in the batch");
     if (ctxs[a]->device != ctxs[0]->device) return fail(ctxs[0], MVR_ERR_BAD_ARG, "the contexts of a batch must share a device");
   }
   mvr_ctx* ctx = ctxs[0];   // the lead: CK() reports into it, its stream runs the batch, its profile records the launches
@@ -1685,7 +1736,7 @@ int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const flo
   const cudaStream_t S = ctx->stream;
   cudaEvent_t ev = get_event(ctx);
   if (!ev) return fail(ctx, MVR_ERR_CUDA, "cudaEventCreate failed");
-  struct Todo { mvr_ctx* m; int slot; NormalsJob job; };
+  struct Todo { mvr_ctx* m; int slot; bool tgt; NormalsJob job; };
   std::vector<Todo> todo;
   std::vector<BuildJob> builds;
   int rc = MVR_OK;
@@ -1695,18 +1746,21 @@ int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const flo
       if (cudaEventRecord(ev, m->stream) != cudaSuccess || cudaStreamWaitEvent(S, ev, 0) != cudaSuccess) rc = fail(ctx, MVR_ERR_CUDA, "stream ordering failed");
     }
     if (rc) break;
-    Cloud& t = m->tgt;
-    if (t.gen == 0) { statuses[a] = fail(m, MVR_ERR_NO_INPUT, "target not set"); continue; }
+    const bool tgt = which_of(a) == MVR_CLOUD_TARGET;
+    Cloud& t = tgt ? m->tgt : m->src;
+    if (t.gen == 0) { statuses[a] = fail(m, MVR_ERR_NO_INPUT, tgt ? "target not set" : "source not set"); continue; }
     statuses[a] = MVR_OK;
     if (t.n == 0) continue;
     uint32_t cells = 0;
     const PairGrid g = normals_grid(m, t, k, &cells);
     BuildJob bj;
-    m->nq.valid = false;
-    if ((rc = plan_pair_index(m, m->nq, 1, t.pts, t.n, t.n_bad, nullptr, g, cells, false, S, &bj))) { ctx->err = m->err; break; }
-    if (m->normals.ensure((size_t)t.n * sizeof(float4)) != cudaSuccess) { rc = fail(ctx, MVR_ERR_CUDA, "normals buffer allocation failed"); break; }
+    PairIndex& ix = tgt ? m->nq : m->nt;
+    ix.valid = false;
+    if ((rc = plan_pair_index(m, ix, tgt ? 1 : 0, t.pts, t.n, t.n_bad, nullptr, g, cells, false, S, &bj))) { ctx->err = m->err; break; }
+    DevBuf& nb = tgt ? m->normals : m->snormals;
+    if (nb.ensure((size_t)t.n * sizeof(float4)) != cudaSuccess) { rc = fail(ctx, MVR_ERR_CUDA, "normals buffer allocation failed"); break; }
     builds.push_back(bj);
-    todo.push_back(Todo{m, a, normals_job(m->nq, t.n, viewpoints ? viewpoints + 3 * a : nullptr, m->normals.as<float4>(), nullptr)});
+    todo.push_back(Todo{m, a, tgt, normals_job(ix, t.n, viewpoints ? viewpoints + 3 * a : nullptr, nb.as<float4>(), nullptr)});
   }
   if (rc == MVR_OK) rc = run_pair_builds(ctx, builds.data(), (int)builds.size(), S);
   for (size_t t0 = 0; rc == MVR_OK && t0 < todo.size(); t0 += BUILD_MAX_JOBS) {
@@ -1721,11 +1775,11 @@ int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const flo
   bool copies = false;
   for (size_t a = 0; rc == MVR_OK && a < todo.size(); ++a) {
     mvr_ctx* m = todo[a].m;
-    m->nq.valid = false;
-    m->has_normals = true;
+    (todo[a].tgt ? m->nq : m->nt).valid = false;
+    (todo[a].tgt ? m->tnrm : m->snrm) = todo[a].job.out;
     float* out = out_nxyzc ? out_nxyzc[todo[a].slot] : nullptr;
     if (!out) continue;
-    if (cudaMemcpyAsync(out, m->normals.p, (size_t)m->tgt.n * sizeof(float4), cudaMemcpyDeviceToHost, S) != cudaSuccess) rc = fail(ctx, MVR_ERR_CUDA, "normals copy failed");
+    if (cudaMemcpyAsync(out, todo[a].job.out, (size_t)todo[a].job.n * sizeof(float4), cudaMemcpyDeviceToHost, S) != cudaSuccess) rc = fail(ctx, MVR_ERR_CUDA, "normals copy failed");
     copies = true;
   }
   // every context's later work waits for the normals (also after a failure: nothing queued above may overlap it)
@@ -1737,6 +1791,12 @@ int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const flo
   ctx->ev_pool.push_back(ev);
   if (rc == MVR_OK && copies) CK(cudaStreamSynchronize(S));
   return rc;
+}
+
+extern "C" {
+
+int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const float* viewpoints, float* const* out_nxyzc, int* statuses) {
+  return mvr::estimate_normals_batch(ctxs, nullptr, count, k, viewpoints, out_nxyzc, statuses);
 }
 
 }  // extern "C"

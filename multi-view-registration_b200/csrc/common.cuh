@@ -61,6 +61,17 @@ __device__ __forceinline__ float4 xform_pinned(const Mat4f& M, float4 p) {
   return r;
 }
 
+// The same without the translation term, for a normal {nx, ny, nz, curvature}: the curvature lane is carried unchanged
+// (transformPointCloudWithNormals).
+__device__ __forceinline__ float4 rotate_pinned(const Mat4f& M, float4 n) {
+  float4 r;
+  r.x = __fadd_rn(__fadd_rn(__fmul_rn(M.m[0], n.x), __fmul_rn(M.m[4], n.y)), __fmul_rn(M.m[8], n.z));
+  r.y = __fadd_rn(__fadd_rn(__fmul_rn(M.m[1], n.x), __fmul_rn(M.m[5], n.y)), __fmul_rn(M.m[9], n.z));
+  r.z = __fadd_rn(__fadd_rn(__fmul_rn(M.m[2], n.x), __fmul_rn(M.m[6], n.y)), __fmul_rn(M.m[10], n.z));
+  r.w = n.w;
+  return r;
+}
+
 __device__ __forceinline__ bool finite3(float4 p) { return isfinite(p.x) && isfinite(p.y) && isfinite(p.z); }
 
 __host__ __device__ __forceinline__ uint32_t part1by2(uint32_t v) {

@@ -1,4 +1,5 @@
-// icp.cu -- per-iteration ICP kernels (the search itself is in pair_search.cuh): estimator sums (K6 point-to-point 3x3 cross-covariance, K9 point-to-plane 6x6 normal equations)
+// icp.cu -- per-iteration ICP kernels (the search itself is in pair_search.cuh): estimator sums (K6 point-to-point 3x3 cross-covariance, K9 point-to-plane and
+// symmetric point-to-plane 6x6 normal equations)
 // with the solve and the convergence test in the reduction's last block, fitness reduction (K8) and
 // order-preserving correspondence compaction.
 //
@@ -191,6 +192,8 @@ __device__ __forceinline__ void icp_advance_frame(IcpState* st, const double (&T
 
 // The tail of one ICP iteration, run by one thread: estimate the increment from the sums, compose it
 // into the accumulated transform, log, and evaluate DefaultConvergenceCriteria (SURVEY.md A8).
+// SYM: the symmetric objective's increment (a separate instance: the others compile as they did before it existed).
+template <bool SYM>
 __device__ __noinline__ void icp_finish_iteration(IcpState* st, IterRec* log) {
   // everything the step needs, fetched up front so the loads overlap (st lives in global memory)
   double S[REDUCE_MAX_VALS], F0[16];
@@ -198,7 +201,7 @@ __device__ __noinline__ void icp_finish_iteration(IcpState* st, IterRec* log) {
   for (int k = 0; k < REDUCE_MAX_VALS; ++k) S[k] = st->sums[k];
 #pragma unroll
   for (int k = 0; k < 16; ++k) F0[k] = st->fin[k];
-  const bool p2l = st->p2l != 0;
+  const bool p2l = st->p2l != 0;   // 0 point-to-point, 1 point-to-plane, 2 symmetric point-to-plane (SYM)
   const double ox = st->ox, oy = st->oy, oz = st->oz;
   const int min_corr = st->min_corr, max_iter = st->max_iter, fixed = st->fixed, iter0 = st->iter;
   const double prev_mse = st->prev_mse, rot_thr = st->rot_thr, trans_thr = st->trans_thr, fit_eps = st->fit_eps;
@@ -216,7 +219,8 @@ __device__ __noinline__ void icp_finish_iteration(IcpState* st, IterRec* log) {
       for (int c = a; c < 6; ++c) { A[a * 6 + c] = S[k]; A[c * 6 + a] = S[k]; ++k; }
     for (int a = 0; a < 6; ++a) b[a] = S[21 + a];
     if (!cholesky_solve6(A, b, x)) { st->reason = 5; st->status = 5; st->done = 1; return; }
-    pose_from_6(x, T);
+    if constexpr (SYM) pose_from_6_symmetric(x, T);
+    else pose_from_6(x, T);
   } else {
     const double inv = 1.0 / cnt;
     const double mu_a[3] = {S[1] * inv, S[2] * inv, S[3] * inv}, mu_b[3] = {S[4] * inv, S[5] * inv, S[6] * inv};
@@ -328,6 +332,29 @@ __device__ __forceinline__ void acc_p2l(double (&v)[REDUCE_P2L_VALS], float4 s, 
   v[28] += (double)d2;
 }
 
+// Symmetric point-to-plane normal equations (TransformationEstimationSymmetricPointToPlaneLLS), the layout of acc_p2l:
+// n = n1 + n2 when n1.n2 >= 0, else n1 - n2 (enforce_same_direction_normals), v = [cross(s + t, n), n], r = n.(t - s).
+// A pair whose n is not finite adds nothing to the system but still counts (and its d2 still enters the mse).
+__device__ __forceinline__ void acc_sym(double (&v)[REDUCE_P2L_VALS], float4 s, float4 t, float4 n1, float4 n2, float d2) {
+  const double sx = s.x, sy = s.y, sz = s.z, tx = t.x, ty = t.y, tz = t.z;
+  const double ax = n1.x, ay = n1.y, az = n1.z, bx = n2.x, by = n2.y, bz = n2.z;
+  const bool same = (ax * bx + ay * by) + az * bz >= 0.0;
+  const double nx = same ? ax + bx : ax - bx, ny = same ? ay + by : ay - by, nz = same ? az + bz : az - bz;
+  v[27] += 1.0;
+  v[28] += (double)d2;
+  if (!(isfinite(nx) && isfinite(ny) && isfinite(nz))) return;
+  const double px = sx + tx, py = sy + ty, pz = sz + tz;
+  const double J[6] = {py * nz - pz * ny, pz * nx - px * nz, px * ny - py * nx, nx, ny, nz};
+  const double r = (nx * (tx - sx) + ny * (ty - sy)) + nz * (tz - sz);
+  int k = 0;
+#pragma unroll
+  for (int a = 0; a < 6; ++a)
+#pragma unroll
+    for (int b = a; b < 6; ++b) v[k++] += J[a] * J[b];
+#pragma unroll
+  for (int a = 0; a < 6; ++a) v[21 + a] += J[a] * r;
+}
+
 // block_reduce_store + last_block_done in one: the block's partial is written, fenced and the ticket drawn by warp 0 alone
 // (the threads that wrote are the ones that fence), so the block's tail is two barriers instead of three and seven warps
 // skip the memory fence.  Same sums in the same order.
@@ -366,23 +393,27 @@ __device__ __forceinline__ bool block_reduce_ticket(double (&v)[NV], double* __r
 }
 
 // Block partials -> (last block) ordered total -> solve, compose, criteria.
-template <int NV>
+template <int NV, bool SYM = false>
 __device__ __forceinline__ void reduce_and_finish(double (&v)[NV], double* __restrict__ partials, IcpState* __restrict__ st,
                                                   IterRec* __restrict__ log, int nblk) {
   if (!block_reduce_ticket<NV>(v, partials, &st->ticket, (unsigned int)nblk)) return;
   ordered_total<NV>(partials, nblk, st->sums);
   if (threadIdx.x == 0) {
     const long long t0 = clock64();
-    icp_finish_iteration(st, log);
+    icp_finish_iteration<SYM>(st, log);
     st->dbg[0] += clock64() - t0; st->dbg[1] += 1;
   }
 }
 
-template <int EST> struct EstVals { static constexpr int value = EST == EST_P2L ? (int)REDUCE_P2L_VALS : (EST == EST_MOM ? (int)REDUCE_MOM_VALS : (int)REDUCE_P2P_VALS); };
+template <int EST> struct EstVals {
+  static constexpr int value = (EST == EST_P2L || EST == EST_SYM) ? (int)REDUCE_P2L_VALS : (EST == EST_MOM ? (int)REDUCE_MOM_VALS : (int)REDUCE_P2P_VALS);
+};
 
+// ns: the source point's normal (symmetric only; read by nothing else)
 template <int EST, int NV>
-__device__ __forceinline__ void acc_pair(double (&v)[NV], float4 s, float4 t, const float4* __restrict__ nrm, float d2, double ox, double oy, double oz) {
-  if constexpr (EST == EST_P2L) acc_p2l(v, s, t, __ldg(nrm + __float_as_int(t.w)), d2);
+__device__ __forceinline__ void acc_pair(double (&v)[NV], float4 s, float4 t, const float4* __restrict__ nrm, const float4* ns, float d2, double ox, double oy, double oz) {
+  if constexpr (EST == EST_SYM) acc_sym(v, s, t, *ns, __ldg(nrm + __float_as_int(t.w)), d2);
+  else if constexpr (EST == EST_P2L) acc_p2l(v, s, t, __ldg(nrm + __float_as_int(t.w)), d2);
   else if constexpr (EST == EST_MOM) acc_mom(v, s, t, d2, ox, oy, oz);
   else acc_p2p(v, s, t, d2, ox, oy, oz);
 }
@@ -441,6 +472,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? MVR_FWD_MINBLOCKS : MV
       p = xform_pinned(M, p);
       p.w = w;
       a.cur[i] = p;
+      if constexpr (EST == EST_SYM) a.nsrc[i] = rotate_pinned(M, a.nsrc[i]);   // the source normals move with the source
     }
     NnBest b;
     fwd_seed(a, i, p, b);
@@ -470,9 +502,9 @@ __global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? MVR_FWD_MINBLOCKS : MV
       if (j < 0) continue;
       const float4 p = a.cur[i];
       const float4 t = __ldg(a.tgt + j);
-      acc_pair<EST>(v, p, t, a.nrm, d2_pinned(p.x, p.y, p.z, t.x, t.y, t.z), ox, oy, oz);
+      acc_pair<EST>(v, p, t, a.nrm, a.nsrc + i, d2_pinned(p.x, p.y, p.z, t.x, t.y, t.z), ox, oy, oz);
     }
-    reduce_and_finish<NV>(v, a.partials, st, a.log, a.grid);
+    reduce_and_finish<NV, EST == EST_SYM>(v, a.partials, st, a.log, a.grid);
   }
 }
 
@@ -558,9 +590,9 @@ __global__ void __launch_bounds__(FUSED_THREADS, MVR_REV_MINBLOCKS * (256 / FUSE
     if (r < 0) continue;
     const float4 t = __ldg(a.tgt + s_q[k]);
     const float4 s = a.cur[r];
-    acc_pair<EST>(v, s, t, a.nrm, d2_pinned(t.x, t.y, t.z, s.x, s.y, s.z), ox, oy, oz);
+    acc_pair<EST>(v, s, t, a.nrm, a.nsrc + r, d2_pinned(t.x, t.y, t.z, s.x, s.y, s.z), ox, oy, oz);
   }
-  reduce_and_finish<NV>(v, a.partials, st, a.log, a.grid);
+  reduce_and_finish<NV, EST == EST_SYM>(v, a.partials, st, a.log, a.grid);
 }
 #endif   // MVR_TS_TILE
 
@@ -612,10 +644,13 @@ cudaError_t launch_icp_forward(const FwdBatch& d_batch, int pairs, int max_grid,
   set_carveout_once();
   const dim3 grid((unsigned)max_grid, (unsigned)pairs);
   if (reciprocal) {
-    // the reciprocal forward half accumulates nothing: one instantiation serves every estimator
-    k_icp_forward<true, EST_P2P><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
+    // the reciprocal forward half accumulates nothing: one instantiation serves every estimator but the symmetric one, whose
+    // source normals move with the source
+    if (est == EST_SYM) k_icp_forward<true, EST_SYM><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
+    else k_icp_forward<true, EST_P2P><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
   } else {
-    if (est == EST_P2L) k_icp_forward<false, EST_P2L><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
+    if (est == EST_SYM) k_icp_forward<false, EST_SYM><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
+    else if (est == EST_P2L) k_icp_forward<false, EST_P2L><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
     else if (est == EST_MOM) k_icp_forward<false, EST_MOM><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
     else k_icp_forward<false, EST_P2P><<<grid, FUSED_THREADS, 0, s>>>(d_batch, first);
   }
@@ -626,7 +661,8 @@ cudaError_t launch_icp_forward(const FwdBatch& d_batch, int pairs, int max_grid,
 cudaError_t launch_icp_reverse(const RevBatch& d_batch, int pairs, int max_grid, int est, cudaStream_t s) {
   if (pairs <= 0 || pairs > FUSED_MAX_PAIRS) return pairs <= 0 ? cudaSuccess : cudaErrorInvalidValue;
   const dim3 grid((unsigned)max_grid, (unsigned)pairs);
-  if (est == EST_P2L) k_icp_reverse<EST_P2L><<<grid, FUSED_THREADS, 0, s>>>(d_batch);
+  if (est == EST_SYM) k_icp_reverse<EST_SYM><<<grid, FUSED_THREADS, 0, s>>>(d_batch);
+  else if (est == EST_P2L) k_icp_reverse<EST_P2L><<<grid, FUSED_THREADS, 0, s>>>(d_batch);
   else if (est == EST_MOM) k_icp_reverse<EST_MOM><<<grid, FUSED_THREADS, 0, s>>>(d_batch);
   else k_icp_reverse<EST_P2P><<<grid, FUSED_THREADS, 0, s>>>(d_batch);
   count_launch();
@@ -672,6 +708,11 @@ __global__ void __launch_bounds__(256) k_align_init(const __grid_constant__ Init
   const int stride = gridDim.x * blockDim.x;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) corr_p[i] = -1;           // no seed yet
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += stride) rmin[i] = 0x7f800000u;   // +inf: "chosen by nobody"
+  if (j.nsrc) {   // symmetric: the source normals by sorted position, turned by the guess like the points were
+    const int nv = j.n_valid;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += stride)
+      j.nsrc[i] = rotate_pinned(j.M, __ldg(j.snrm + __float_as_int(__ldg(j.sorted + i).w)));
+  }
   if (blockIdx.x == 0) {
     static_assert(sizeof(IcpState) % 4 == 0, "IcpState words");
     const uint32_t* src = reinterpret_cast<const uint32_t*>(stage + blockIdx.y);

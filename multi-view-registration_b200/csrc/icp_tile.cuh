@@ -49,6 +49,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? MVR_FWD_MINBLOCKS : MV
         p = xform_pinned(M, p);
         p.w = w;
         a.cur[i] = p;
+        if constexpr (EST == EST_SYM) a.nsrc[i] = rotate_pinned(M, a.nsrc[i]);
       }
       me.qx = p.x; me.qy = p.y; me.qz = p.z;
       fwd_seed(a, i, p, me.b);
@@ -126,9 +127,9 @@ __global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? MVR_FWD_MINBLOCKS : MV
       if (j < 0) continue;
       const float4 p = a.cur[i];
       const float4 t = __ldg(a.tgt + j);
-      acc_pair<EST>(v, p, t, a.nrm, d2_pinned(p.x, p.y, p.z, t.x, t.y, t.z), ox, oy, oz);
+      acc_pair<EST>(v, p, t, a.nrm, a.nsrc + i, d2_pinned(p.x, p.y, p.z, t.x, t.y, t.z), ox, oy, oz);
     }
-    reduce_and_finish<NV>(v, a.partials, st, a.log, a.grid);
+    reduce_and_finish<NV, EST == EST_SYM>(v, a.partials, st, a.log, a.grid);
   }
 }
 
@@ -267,8 +268,8 @@ __global__ void __launch_bounds__(FUSED_THREADS, MVR_REV_MINBLOCKS * (256 / FUSE
     if (r < 0) continue;
     const float4 t = __ldg(a.tgt + s_q[k]);
     const float4 s = a.cur[r];
-    acc_pair<EST>(v, s, t, a.nrm, d2_pinned(t.x, t.y, t.z, s.x, s.y, s.z), ox, oy, oz);
+    acc_pair<EST>(v, s, t, a.nrm, a.nsrc + r, d2_pinned(t.x, t.y, t.z, s.x, s.y, s.z), ox, oy, oz);
   }
-  reduce_and_finish<NV>(v, a.partials, st, a.log, a.grid);
+  reduce_and_finish<NV, EST == EST_SYM>(v, a.partials, st, a.log, a.grid);
 }
 

@@ -83,7 +83,7 @@ struct IcpState {
   double ox, oy, oz;      // origin the sums are taken about
   unsigned long long queries;
   int iter, done, reason, status, n_corr;
-  int max_iter, fixed, min_corr, p2l, recip, n_src;
+  int max_iter, fixed, min_corr, p2l, recip, n_src;   // p2l: estimator of the solve, 0 point-to-point, 1 point-to-plane, 2 symmetric
   unsigned int ticket;    // blocks of the running reduction that have finished
   long long dbg[8];       // diagnostics: [0] clock cycles spent in the serial solve, [1] solves, [2] reciprocal searches that lost their chooser (must be 0),
                           // [3] forward queries answered by the per-thread fallback, [4] forward rounds whose tile did not fit,
@@ -155,6 +155,7 @@ struct FwdArgs {
   IcpState* st;
   IterRec* log;
   int grid;                // blocks that work on this pair (a pure function of the cloud size): fused_grid(n_valid)
+  float4* nsrc;            // source normals by SORTED position, current orientation (updated in place; symmetric only)
 };
 struct RevArgs {
   const float4* tgt;
@@ -172,9 +173,10 @@ struct RevArgs {
   IterRec* log;
   int grid;                // fused_grid_rev(m_valid)
   int per;                 // fused_rev_chunks(m_valid): chunks of 256 target points per block (<= 4)
+  const float4* nsrc;      // = FwdArgs::nsrc
 };
 // est: which sums the iteration accumulates over its correspondences
-enum { EST_P2P = 0, EST_P2L = 1, EST_MOM = 2 /* point-to-point + second moments (LUM edge statistics) */ };
+enum { EST_P2P = 0, EST_P2L = 1, EST_MOM = 2 /* point-to-point + second moments (LUM edge statistics) */, EST_SYM = 3 /* symmetric point-to-plane */ };
 // One launch advances EVERY pair of a group by one iteration half: blockIdx.y selects the pair, blockIdx.x < grid of
 // that pair does its work.  The arguments of all pairs travel by value in the kernel's parameter (constant) space, so
 // indexing them by pair costs no registers.  max_grid = the largest grid of the group.
@@ -182,11 +184,19 @@ enum { EST_P2P = 0, EST_P2L = 1, EST_MOM = 2 /* point-to-point + second moments 
 enum { FUSED_MAX_PAIRS = 24 };
 struct FwdBatch { FwdArgs a[FUSED_MAX_PAIRS]; };
 struct RevBatch { RevArgs a[FUSED_MAX_PAIRS]; };
+// kernel parameter space (sm_70 and later, CUDA >= 12.1): 32764 bytes
+static_assert(sizeof(FwdBatch) + sizeof(int) <= 32764 && sizeof(RevBatch) <= 32764, "a group's arguments must fit the kernel parameters");
 // Start of a batch of aligns in one launch: per pair, corr_p <- -1 (no seed), rmin <- +inf bits (chosen by nobody; nullable),
 // *st <- stage[k] (the initial states, uploaded together).  End of a batch: stage[k] <- *st (dbg[3] of the copy = the pair's
-// crowded word, which is reset).
-struct InitJob { int32_t* corr_p; int n; int m; uint32_t* rmin; IcpState* st; uint32_t* crowded; };
+// crowded word, which is reset).  Symmetric aligns (nsrc non-null) also get their source normals by sorted position:
+// nsrc[i] <- R(M) snrm[sorted[i].w] for the n_valid finite source points (the guess's rotation, pinned; curvature kept).
+struct InitJob {
+  int32_t* corr_p; int n; int m; uint32_t* rmin; IcpState* st; uint32_t* crowded;
+  float4* nsrc; const float4* snrm; const float4* sorted; int n_valid; int pad_;
+  Mat4f M;
+};
 struct InitBatch { InitJob j[BUILD_MAX_JOBS]; };
+static_assert(sizeof(InitBatch) + sizeof(void*) <= 32764, "the batch's jobs must fit the kernel parameters");
 cudaError_t launch_align_init(const InitBatch& batch, int count, const IcpState* stage, cudaStream_t s);
 cudaError_t launch_align_gather(const InitBatch& batch, int count, IcpState* stage, cudaStream_t s);
 int fused_grid(int items);

@@ -190,6 +190,18 @@ MVR_HD inline void pose_from_6(const double* x, double* T) {
   }
 }
 
+// The increment of the symmetric objective (TransformationEstimationSymmetricPointToPlaneLLS::constructTransformationMatrix):
+// T = R Trans(x3, x4, x5) R with the R of pose_from_6, i.e. rotation R R and translation R t.  Column-major 4x4.
+MVR_HD inline void pose_from_6_symmetric(const double* x, double* T) {
+  double R[16];
+  pose_from_6(x, R);   // R[c * 4 + r]; its translation column is t
+  for (int k = 0; k < 16; ++k) T[k] = (k % 5 == 0) ? 1.0 : 0.0;
+  for (int r = 0; r < 3; ++r) {
+    for (int c = 0; c < 3; ++c) T[c * 4 + r] = (R[r] * R[c * 4] + R[4 + r] * R[c * 4 + 1]) + R[8 + r] * R[c * 4 + 2];
+    T[12 + r] = (R[r] * x[3] + R[4 + r] * x[4]) + R[8 + r] * x[5];
+  }
+}
+
 // Symmetric 3x3 eigen-decomposition by cyclic Jacobi (row-major C), eigenvalues ascending,
 // eigenvectors in the columns of V (row-major).
 MVR_HD inline void eig_sym3(const double* C, double* w, double* V) {

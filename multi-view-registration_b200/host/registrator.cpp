@@ -437,19 +437,35 @@ int Registrator::multiViewRegister(std::vector<View>& views, const mvr_turntable
   }
   const double t_set = now();
   // the source of pair p is the view that pair p + 1 has as its target: shared, not measured again
+  std::vector<int> src_of((size_t)P);   // the context whose target is pair k's source view, if this rank has that pair (else >= P)
   for (int k = 0; k < P; ++k) {
     const int sv = (p0 + k + 1) % V;
-    const int j = ((sv - p0) % V + V) % V;   // the context whose target is view sv, if this rank has that pair
+    const int j = ((sv - p0) % V + V) % V;
+    src_of[(size_t)k] = j;
     if (j < P) rc = mvr_cloud_share(ctx_[(size_t)k], MVR_CLOUD_SOURCE, ctx_[(size_t)j], MVR_CLOUD_TARGET);
     else rc = mvr_set_source_device(ctx_[(size_t)k], dview[(size_t)sv], views[(size_t)sv].size);
     if (rc) return fail(rc, mvr_last_error(ctx_[(size_t)k]));
   }
-  // point-to-plane: the target normals of every pair in one batch, each towards the origin of its view's own sensor frame (PCL's
-  // default viewpoint); a pure function of the view, so pair poses do not depend on how the ring is sharded.  The repeats
-  // reuse them; a source (shared or not) needs none.
-  if (prm.icp.estimator == MVR_POINT_TO_PLANE) {
-    if ((rc = mvr_estimate_normals_batch(cs.data(), P, normal_k, nullptr, nullptr, st.data()))) return fail(rc, mvr_last_error(cs[0]));
-    for (int k = 0; k < P; ++k) if (st[(size_t)k]) return fail(st[(size_t)k], mvr_last_error(cs[(size_t)k]));
+  // point-to-plane and symmetric: the target normals of every pair in one batch, each towards the origin of its view's own sensor
+  // frame (PCL's default viewpoint); a pure function of the view, so pair poses do not depend on how the ring is sharded.  The
+  // repeats reuse them.  Point-to-plane needs no source normals.  Symmetric: a source view that is a target here shares that
+  // pair's normals; the one that is not (the last source of a pair range) is estimated in the same batch -- the same grid and
+  // kernel, so the same bits as on the rank that has it as a target.
+  const bool sym = prm.icp.estimator == MVR_SYMMETRIC;
+  if (prm.icp.estimator == MVR_POINT_TO_PLANE || sym) {
+    std::vector<mvr_ctx*> nc(cs);
+    std::vector<int> nw((size_t)P, MVR_CLOUD_TARGET);
+    if (sym)
+      for (int k = 0; k < P; ++k)
+        if (src_of[(size_t)k] >= P) { nc.push_back(cs[(size_t)k]); nw.push_back(MVR_CLOUD_SOURCE); }
+    std::vector<int> nst(nc.size(), 0);
+    if ((rc = estimate_normals_batch(nc.data(), nw.data(), (int)nc.size(), normal_k, nullptr, nullptr, nst.data()))) return fail(rc, mvr_last_error(cs[0]));
+    for (size_t a = 0; a < nc.size(); ++a) if (nst[a]) return fail(nst[a], mvr_last_error(nc[a]));
+    for (int k = 0; sym && k < P; ++k) {
+      const int j = src_of[(size_t)k];
+      if (j >= P || views[(size_t)((p0 + k + 1) % V)].size == 0) continue;   // an empty view has no normals; its pairs report MVR_ERR_NO_INPUT
+      if ((rc = mvr_normals_share(cs[(size_t)k], MVR_CLOUD_SOURCE, cs[(size_t)j], MVR_CLOUD_TARGET))) return fail(rc, mvr_last_error(cs[(size_t)k]));
+    }
   }
   const double t_share = now();
   const int repeats = std::max(prm.repeat_times, 1);

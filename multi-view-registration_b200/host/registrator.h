@@ -173,4 +173,9 @@ int lumRelax(const std::vector<mvr_pair_moments>& edges, const int* src, const i
 bool leastSquares(const std::vector<double>& A, const std::vector<double>& b, int rows, int cols, std::vector<double>& x);
 int refineAxisFromPoses(const std::vector<Matrix4d>& poses, double pivot[3], double axis[3]);
 
+// mvr_estimate_normals_batch with a cloud per entry (api.cu; not part of the C ABI): which[k] (mvr_cloud) picks the target or
+// the source normals of ctxs[k], kept as that cloud's normals; a context may appear once per cloud.  which = NULL: all targets.
+int estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int count, int k, const float* viewpoints, float* const* out_nxyzc,
+                           int* statuses);
+
 }  // namespace mvr

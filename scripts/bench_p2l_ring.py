@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""Point-to-point vs point-to-plane turntable ring registration on one GPU (DESIGN.md section 7).
+"""Point-to-point vs point-to-plane vs symmetric point-to-plane turntable ring registration on one GPU (DESIGN.md section 7).
 
 Workload: 24 views x 200k points (synth.turntable_sequence), scans resident on the device, reciprocal correspondences, max_dist 4,
 loop closure on, the bench's initial guesses (ideal turntable pose, the fixed perturbation on every odd view).  In one process,
-after a warm-up, the two estimators alternate; the script reports
+after a warm-up, the three estimators alternate; the script reports
 
   ring_ms        ms per register_turntable call (30 fixed iterations; host clock around the call and a device synchronise,
                  L2 overwritten before each call), median and spread over --steps calls per estimator
@@ -77,7 +77,7 @@ def main():
 
     reg = mvr.Registrator(0, 1)
     bound = reg.bind_views([(t.data_ptr(), n) for t in d_views], init)
-    names = {mvr.POINT_TO_POINT: "point_to_point", mvr.POINT_TO_PLANE: "point_to_plane"}
+    names = {mvr.POINT_TO_POINT: "point_to_point", mvr.POINT_TO_PLANE: "point_to_plane", mvr.SYMMETRIC: "symmetric"}
 
     def params(est, fixed=True, max_iterations=None, eps=0.0):
         icp = mvr.default_params(max_iterations=max_iterations or a.iters, max_dist=4.0, reciprocal=1, fixed_iterations=1 if fixed else 0,
