@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 HOST = os.path.join(HERE, "host")
 LIB = os.path.join(HERE, "libmvr_b200.so")
 
-CU_SOURCES = ["index.cu", "bin.cu", "pair_index.cu", "cell_nn.cu", "icp.cu", "normals.cu", "denoise.cu", "api.cu"]
+CU_SOURCES = ["index.cu", "pair_index.cu", "cell_nn.cu", "icp.cu", "normals.cu", "denoise.cu", "api.cu"]
 HOST_SOURCES = ["registrator.cpp", "lum.cpp", "capi.cpp", "multi.cpp"]
 
 NVCC_FLAGS = [
@@ -57,8 +57,7 @@ def stale():
 def build(force=False, verbose=False, out=None):
     if out is None and not force and not stale():
         return LIB
-    extra = os.environ.get("MVR_NVCC_DEFS", "").split()   # development: e.g. MVR_NVCC_DEFS="-DMVR_BS_THREADS=64"
-    cmd = [_nvcc()] + NVCC_FLAGS + extra + ["-shared", "-o", out or LIB, "-x", "cu"] + sources() + ["-ldl"]
+    cmd = [_nvcc()] + NVCC_FLAGS + ["-shared", "-o", out or LIB, "-x", "cu"] + sources() + ["-ldl"]
     if verbose:
         cmd += ["-Xptxas", "-v"]
         print(" ".join(cmd))

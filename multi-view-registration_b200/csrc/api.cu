@@ -21,12 +21,10 @@
 #include "launch.h"
 #include "small_solve.h"
 
-// x cells per y/z cell edge of the per-align indices of the fused ICP iteration (pair_search.cuh); measured in DESIGN.md section 7
-#ifndef MVR_PG_XRATIO
-#define MVR_PG_XRATIO 4
-#endif
-
 using namespace mvr;
+
+// x cells per y/z cell edge of the per-align indices of the fused ICP iteration (pair_search.cuh); measured in DESIGN.md section 7
+constexpr int PG_XRATIO = 4;
 
 #include <atomic>
 namespace mvr {
@@ -63,25 +61,19 @@ struct Cloud {
   float lo[3] = {0, 0, 0}, hi[3] = {0, 0, 0};
   int n_bad = 0;
   uint64_t gen = 0;
-  // index: `sorted` (cell-ordered points, .w = original index) + `table` (cell starts).  Built either by
-  // the counting sort of bin.cu (order inside a cell unspecified) or by the stable radix sort of
-  // index.cu (mvr_index_build; `exportable`, keys/perm kept for mvr_index_export).
+  // index: `sorted` (cell-ordered points, .w = original index) + `table` (cell starts), built by the stable
+  // radix sort of index.cu (mvr_index_build; `exportable`, keys/perm kept for mvr_index_export).
   bool index_valid = false;
   bool exportable = false;
   uint64_t index_gen = 0;
   mvr_grid grid{};
   GridDev gd{};
-  DevBuf keys, vals, keys_alt, vals_alt, hist, counters, sorted, table;
+  DevBuf keys, vals, keys_alt, vals_alt, hist, sorted, table;
   uint32_t* sorted_keys = nullptr;
   uint32_t* perm = nullptr;
-  IndexDev dev() const {
-    IndexDev ix;
-    ix.pts = sorted.as<float4>(); ix.start = table.as<uint32_t>(); ix.g = gd; ix.n_valid = n - n_bad;
-    return ix;
-  }
   void release() {
     own.release(); keys.release(); vals.release(); keys_alt.release(); vals_alt.release(); hist.release();
-    counters.release(); sorted.release(); table.release();
+    sorted.release(); table.release();
   }
 };
 
@@ -89,7 +81,7 @@ struct ProfRec { int kind; cudaEvent_t a, b; double bytes, units; int count; };
 
 // Per-align row-major index of one cloud (pair_index.cu).
 struct PairIndex {
-  DevBuf sorted, start, s0;   // points by cell (the source's move in place), cell table, source binning-time copy
+  DevBuf sorted, start;       // points by cell (the source's move in place), cell table
   DevBuf gocc, gmask;         // gate mask of a target index (pair_index.cu) and its undilated occupancy words
   float gm_gate = -1.f;       // the gate (float d2, rounded up) the mask was built for; < 0: none
   int gm_stride = 0;
@@ -98,7 +90,7 @@ struct PairIndex {
   int n_valid = 0;
   uint64_t gen = 0;
   bool valid = false;
-  void release() { sorted.release(); start.release(); s0.release(); gocc.release(); gmask.release(); gm_gate = -1.f; valid = false; }
+  void release() { sorted.release(); start.release(); gocc.release(); gmask.release(); gm_gate = -1.f; valid = false; }
 };
 
 }  // namespace
@@ -115,11 +107,10 @@ struct mvr_ctx {
   const float4* snrm = nullptr;
   DevBuf nsrc;                   // symmetric aligns: the source normals by sorted position, moved with the source
   Mat4f guess_m{};               // the guess of the prepared align (turns the source normals at its start)
-  DevBuf cur, corr_p, corr_j, corr_d2, rmin, rnn, partials, sums, out_cloud, qtmp, itmp, ftmp, scratch, misc, tiles, state, log;
+  DevBuf corr_p, corr_j, corr_d2, rmin, rnn, partials, sums, out_cloud, qtmp, itmp, ftmp, scratch, misc, state, log;
   PairIndex pt, ps;              // target / source index of the running align
   PairIndex nt, nq;              // target / query index of the dense NN pass (cell_nn.cu)
   double nn_ppc = 8.0;           // its target points per occupied cell
-  double nn_dense_ratio = 8.0;   // kept for mvr_ctx_set_nn_options (unused: batches above nn_sorted_from are sorted and seeded)
   int nn_mode = MVR_NN_AUTO;     // mvr_ctx_set_nn_mode
   int nn_sorted_from = 262144;   // AUTO: batches larger than this are sorted by cell and answered by the seeded pass
   bool gate_mask = false;        // mvr_ctx_set_gate_mask
@@ -326,7 +317,7 @@ mvr_grid auto_grid(mvr_ctx* ctx, const Cloud& c) {
 PairGrid make_pair_grid(const float lo[3], const float hi[3], double e, uint32_t* cells_out, int xr = 1);
 bool same_pair_grid(const PairGrid& a, const PairGrid& b);
 int build_pair_index(mvr_ctx* ctx, PairIndex& ix, const float4* pts, int n, int n_bad, const Mat4f* guess, const PairGrid& g,
-                     uint32_t cells, bool keep_s0, bool ordered = true);
+                     uint32_t cells, bool ordered = true);
 int plan_pair_index(mvr_ctx* ctx, PairIndex& ix, int slot, const float4* pts, int n, int n_bad, const Mat4f* guess, const PairGrid& g,
                     uint32_t cells, bool ordered, cudaStream_t stream, BuildJob* job);
 int run_pair_builds(mvr_ctx* ctx, const BuildJob* jobs, int count, cudaStream_t stream);
@@ -343,10 +334,10 @@ int nn_pass_dense(mvr_ctx* ctx, const float4* q, int n, int32_t* d_idx, float* d
   const PairGrid g = make_pair_grid(t.lo, t.hi, e, &cells);
   int rc;
   if (!(ctx->nt.valid && ctx->nt.gen == t.gen && same_pair_grid(ctx->nt.g, g))) {
-    if ((rc = build_pair_index(ctx, ctx->nt, t.pts, t.n, t.n_bad, nullptr, g, cells, false))) return rc;
+    if ((rc = build_pair_index(ctx, ctx->nt, t.pts, t.n, t.n_bad, nullptr, g, cells))) return rc;
     ctx->nt.gen = t.gen;
   }
-  if ((rc = build_pair_index(ctx, ctx->nq, q, n, 0, nullptr, g, cells, false, false))) return rc;
+  if ((rc = build_pair_index(ctx, ctx->nq, q, n, 0, nullptr, g, cells, false))) return rc;
   ProfScope ps(ctx, MVR_K_NN, 24.0 * n + 16.0 * t.n, (double)n);
   if (seeded)
     CK(launch_seeded_nn(ctx->nq.sorted.as<float4>(), n, ctx->nq.start.as<uint32_t>() + cells, ctx->nt.sorted.as<float4>(),
@@ -372,7 +363,7 @@ int nn_pass(mvr_ctx* ctx, const float4* q, int n, int32_t* d_idx, float* d_d2) {
   if (!(pt.valid && pt.gen == t.gen && pt.g.xr == 1.0f)) {   // the NN kernels take isotropic cells
     uint32_t cells = 0;
     const PairGrid gt = make_pair_grid(t.lo, t.hi, pair_cell_edge(ctx, t, INFINITY), &cells);
-    if ((rc = build_pair_index(ctx, pt, t.pts, t.n, t.n_bad, nullptr, gt, cells, false))) return rc;
+    if ((rc = build_pair_index(ctx, pt, t.pts, t.n, t.n_bad, nullptr, gt, cells))) return rc;
     pt.gen = t.gen;
   }
   ProfScope ps(ctx, MVR_K_NN, 24.0 * n + 16.0 * t.n, (double)n);
@@ -386,7 +377,7 @@ int nn_pass(mvr_ctx* ctx, const float4* q, int n, int32_t* d_idx, float* d_d2) {
     return MVR_OK;
   }
   const bool sorted = n > 262144;
-  if (sorted && (rc = build_pair_index(ctx, ctx->nq, q, n, 0, nullptr, pt.g, pt.cells, false, false))) return rc;
+  if (sorted && (rc = build_pair_index(ctx, ctx->nq, q, n, 0, nullptr, pt.g, pt.cells, false))) return rc;
   CK(launch_pair_nn(sorted ? ctx->nq.sorted.as<float4>() : q, n, sorted, pt.sorted.as<float4>(), pt.start.as<uint32_t>(), pt.g, pt.n_valid, d_idx,
                     d_d2, ctx->stream));
   return MVR_OK;
@@ -504,8 +495,7 @@ int run_pair_builds(mvr_ctx* ctx, const BuildJob* jobs, int count, cudaStream_t 
 }
 
 int build_pair_index(mvr_ctx* ctx, PairIndex& ix, const float4* pts, int n, int n_bad, const Mat4f* guess, const PairGrid& g,
-                     uint32_t cells, bool keep_s0, bool ordered) {
-  (void)keep_s0;
+                     uint32_t cells, bool ordered) {
   BuildJob job;
   ix.valid = false;
   int rc = plan_pair_index(ctx, ix, &ix == &ctx->pt || &ix == &ctx->nt ? 0 : 1, pts, n, n_bad, guess, g, cells, ordered, ctx->stream, &job);
@@ -650,8 +640,8 @@ int mvr_ctx_destroy(mvr_ctx* ctx) {
   ctx->stage_dev.release(); ctx->bbox_dev.release();
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_bbox) cudaFreeHost(ctx->h_bbox);
-  DevBuf* bufs[] = {&ctx->cur, &ctx->corr_p, &ctx->rmin, &ctx->rnn, &ctx->corr_j, &ctx->corr_d2, &ctx->partials, &ctx->sums, &ctx->out_cloud, &ctx->qtmp,
-                    &ctx->itmp, &ctx->ftmp, &ctx->scratch, &ctx->misc, &ctx->tiles, &ctx->state, &ctx->log, &ctx->crowded};
+  DevBuf* bufs[] = {&ctx->corr_p, &ctx->rmin, &ctx->rnn, &ctx->corr_j, &ctx->corr_d2, &ctx->partials, &ctx->sums, &ctx->out_cloud, &ctx->qtmp,
+                    &ctx->itmp, &ctx->ftmp, &ctx->scratch, &ctx->misc, &ctx->state, &ctx->log, &ctx->crowded};
   for (DevBuf* b : bufs) b->release();
   if (ctx->h_sums) cudaFreeHost(ctx->h_sums);
   if (ctx->h_small) cudaFreeHost(ctx->h_small);
@@ -711,7 +701,6 @@ int mvr_ctx_set_index_options(mvr_ctx* ctx, float cell_edge, int max_bits) {
 int mvr_ctx_set_nn_options(mvr_ctx* ctx, double points_per_cell, double dense_ratio) {
   if (!ctx || !(points_per_cell > 0) || !(dense_ratio >= 0)) return MVR_ERR_BAD_ARG;
   ctx->nn_ppc = points_per_cell;
-  ctx->nn_dense_ratio = dense_ratio;
   ctx->nt.valid = false;
   return MVR_OK;
 }
@@ -1010,7 +999,7 @@ static int align_plan(mvr_ctx* ctx, const mvr_icp_params* prm, const float* gues
   int rc = MVR_OK;
   {
     uint32_t cells = 0;
-    const PairGrid gt = make_pair_grid(ctx->tgt.lo, ctx->tgt.hi, pair_cell_edge(ctx, ctx->tgt, max_dist), &cells, MVR_PG_XRATIO);
+    const PairGrid gt = make_pair_grid(ctx->tgt.lo, ctx->tgt.hi, pair_cell_edge(ctx, ctx->tgt, max_dist), &cells, PG_XRATIO);
     PairIndex& pt = ctx->pt;
     if (!(pt.valid && pt.gen == ctx->tgt.gen && same_pair_grid(pt.g, gt))) {
       BuildJob job;
@@ -1034,7 +1023,7 @@ static int align_plan(mvr_ctx* ctx, const mvr_icp_params* prm, const float* gues
     for (int a = 0; a < 3; ++a) if (!(lo[a] <= hi[a])) { lo[a] = 0.f; hi[a] = 0.f; }
     uint32_t cells = 0;
     // the cell edge follows the source's own density (its box as given: a rigid guess keeps the surface area)
-    const PairGrid gs = make_pair_grid(lo, hi, pair_cell_edge(ctx, s, max_dist), &cells, MVR_PG_XRATIO);
+    const PairGrid gs = make_pair_grid(lo, hi, pair_cell_edge(ctx, s, max_dist), &cells, PG_XRATIO);
     Mat4f Gm;
     std::memcpy(Gm.m, G, sizeof(Gm.m));
     ctx->guess_m = Gm;
@@ -1222,8 +1211,7 @@ static int align_run(mvr_ctx* const* ctxs, int count, const mvr_icp_params* prm,
   // 8 points 19.85, 16 points 20.1 -- about one point per 600k source points of the batch, at most four.
   long long batch_points = 0;
   for (int k = 0; k < count; ++k) batch_points += ctxs[k]->fa.n_valid;
-  static const int fwd_items_env = [] { const char* e = std::getenv("MVR_FWD_ITEMS"); return e ? std::atoi(e) : 0; }();
-  const int fwd_items = fwd_items_env > 0 ? fwd_items_env : (int)std::min<long long>(4, std::max<long long>(1, (batch_points + 300000) / 600000));
+  const int fwd_items = (int)std::min<long long>(4, std::max<long long>(1, (batch_points + 300000) / 600000));
   std::vector<Group> groups;
   for (int g0 = 0; g0 < count; g0 += gsz) {
     Group g{};
@@ -1654,7 +1642,7 @@ int mvr_denoise(mvr_ctx* ctx, const void* points, size_t n, size_t stride_bytes,
   const PairGrid g = make_pair_grid(tmp.lo, tmp.hi, triangle_length * 1.0001, &cells);
   if ((double)g.cell_lo < triangle_length) return fail(ctx, MVR_ERR_BAD_ARG, "cloud too large for this edge length (grid capped)");
   PairIndex& ix = ctx->nq;
-  if ((rc = build_pair_index(ctx, ix, tmp.pts, ni, tmp.n_bad, nullptr, g, cells, false, false))) return rc;
+  if ((rc = build_pair_index(ctx, ix, tmp.pts, ni, tmp.n_bad, nullptr, g, cells, false))) return rc;
   // parent | count | keys | vals | keys_alt | vals_alt | hist | n_noise
   const size_t nb = (size_t)radix_num_blocks(ni) * 256;
   CK(ctx->itmp.ensure(((size_t)6 * n + nb + 16) * sizeof(uint32_t)));
@@ -1688,7 +1676,7 @@ int mvr_estimate_normals(mvr_ctx* ctx, int which, int k, const float viewpoint[3
   uint32_t cells = 0;
   const PairGrid g = normals_grid(ctx, c, k, &cells);
   PairIndex& ix = ctx->nq;
-  int rc = build_pair_index(ctx, ix, c.pts, n, c.n_bad, nullptr, g, cells, false, false);
+  int rc = build_pair_index(ctx, ix, c.pts, n, c.n_bad, nullptr, g, cells, false);
   if (rc) return rc;
   DevBuf& nb = which == MVR_CLOUD_TARGET ? ctx->normals : ctx->snormals;
   CK(nb.ensure((size_t)n * sizeof(float4)));

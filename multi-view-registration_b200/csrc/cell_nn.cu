@@ -14,7 +14,7 @@
 //     divergence inside a cell;
 //   * the neighbourhood holds the true neighbour whenever the best distance found is smaller than the distance
 //     from the query to the neighbourhood's boundary (checked per query with the conservative cell geometry of
-//     nn_search.cuh); the few queries that fail the test finish with the seeded general search of pair_search.cuh.
+//     pair_search.cuh); the few queries that fail the test finish with the seeded general search of pair_search.cuh.
 //
 // Ties resolve to the lowest original index: the comparison key is (d2 bits, index) as one 64-bit integer.
 // Algorithmic bytes: 16 B per query read + 8 B result, 16 B per target point, 8 B per cell-table entry.
@@ -54,10 +54,8 @@ __device__ __forceinline__ float cn_face(float t, int c, int n, int h) {
   return u;
 }
 
-#ifndef MVR_CN_MINBLOCKS
-#define MVR_CN_MINBLOCKS 4
-#endif
-__global__ void __launch_bounds__(CN_THREADS, MVR_CN_MINBLOCKS) k_cell_nn(CellNnArgs a) {
+constexpr int CN_MINBLOCKS = 4;
+__global__ void __launch_bounds__(CN_THREADS, CN_MINBLOCKS) k_cell_nn(CellNnArgs a) {
   __shared__ float4 s_pts[CN_WARPS][PG_SEGS * 32 / 2];   // 32 staged points per warp; the fallback's segment list (PG_SEGS x 32 uint2) reuses it
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const PairGrid g = a.g;

@@ -20,19 +20,11 @@ struct GridDev {
   int G;
 };
 
-// A Morton-sorted cloud: pts[k] = {x, y, z, bits(original index)}, start has (1<<3*bits)+1 entries.
-struct IndexDev {
-  const float4* pts;
-  const uint32_t* start;
-  GridDev g;
-  int n_valid;   // finite points (they occupy sorted positions [0, n_valid))
-};
-
 // Row-major uniform grid of the per-align index (pair_index.cu): nx x ny x nz cells, x fastest,
 // cell_a = clamp(floor((p_a - o_a) * inv_cell), 0, n_a - 1).
 // Cells may be FINER along x (xr cells per y/z cell edge, xr = 1, 2, 4 or 8): the points of a (y, z) row are one contiguous run
 // whatever the x resolution, so a finer x only narrows the run a ball query reads -- the same two table loads per row, fewer
-// candidates (the fused ICP iteration uses xr = MVR_PG_XRATIO; every other user of the grid builds it with xr = 1).
+// candidates (the fused ICP iteration uses xr = PG_XRATIO of api.cu; every other user of the grid builds it with xr = 1).
 struct PairGrid {
   float ox, oy, oz;
   float inv_cell;     // y and z: cells per unit length

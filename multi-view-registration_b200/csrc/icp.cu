@@ -13,28 +13,17 @@
 
 #include "launch.h"
 #include "pair_search.cuh"
-#ifdef MVR_TS_TILE
-#include "tile_search.cuh"
-#endif
 #include "small_solve.h"
 
+namespace mvr {
+
 // candidates evaluated per trip of the flat scan = independent 16-byte loads in flight per thread (measured: 8 > 4 > 2)
+constexpr int PG_UNROLL = 6;
 // resident 256-thread blocks per SM the register allocation aims at (forward reciprocal half / reverse half);
 // measured on B200, same box, 24 x 200k pairs: (4, 3) 37.5 ms, (5, 3) 36.5, (4, 4) 34.9, (5, 4) 33.9, (5, 5) 34.3, (6, 6) 36.4
-#ifndef MVR_FWD_MINBLOCKS
-#define MVR_FWD_MINBLOCKS 5
-#endif
-#ifndef MVR_FWD1_MINBLOCKS
-#define MVR_FWD1_MINBLOCKS 3   // one-way forward kernel (search + estimator sums)
-#endif
-#ifndef MVR_REV_MINBLOCKS
-#define MVR_REV_MINBLOCKS 4
-#endif
-#ifndef MVR_PG_UNROLL
-#define MVR_PG_UNROLL 6
-#endif
-
-namespace mvr {
+constexpr int FWD_MINBLOCKS = 5;
+constexpr int FWD1_MINBLOCKS = 3;   // one-way forward kernel (search + estimator sums)
+constexpr int REV_MINBLOCKS = 4;
 
 // ---------------------------------------------------------------------------------------------
 // estimator sums: fixed topology (thread grid-stride over ORIGINAL indices -> warp shuffle tree ->
@@ -441,11 +430,8 @@ __device__ __forceinline__ void fwd_commit(const FwdArgs& a, int i, const NnBest
   }
 }
 
-#ifdef MVR_TS_TILE
-#include "icp_tile.cuh"
-#else
 template <bool RECIP, int EST>
-__global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? MVR_FWD_MINBLOCKS : MVR_FWD1_MINBLOCKS) * (256 / FUSED_THREADS)) k_icp_forward(const __grid_constant__ FwdBatch batch, int first) {
+__global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? FWD_MINBLOCKS : FWD1_MINBLOCKS) * (256 / FUSED_THREADS)) k_icp_forward(const __grid_constant__ FwdBatch batch, int first) {
   // this pair's arguments: parameter space -> shared memory (a dynamically indexed parameter would be copied to
   // local memory and pin registers)
   __shared__ FwdArgs s_args;
@@ -483,7 +469,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? MVR_FWD_MINBLOCKS : MV
       const uint32_t wd = __ldg(a.gmask + ((size_t)cz * a.gt.ny + cy) * a.gm_stride + (cx >> 5));
       if (!((wd >> (cx & 31)) & 1u)) { a.corr_p[i] = -1; continue; }
     }
-    pg_search<MVR_PG_UNROLL>(a.gt, a.tstart, a.tgt, a.m_valid, p.x, p.y, p.z, p.x, p.y, p.z, 0.0f, 1.0f, a.max_d2f, b, seg);
+    pg_search<PG_UNROLL>(a.gt, a.tstart, a.tgt, a.m_valid, p.x, p.y, p.z, p.x, p.y, p.z, 0.0f, 1.0f, a.max_d2f, b, seg);
     fwd_commit<RECIP>(a, i, b, ngate);
   }
   if (RECIP) {
@@ -512,12 +498,9 @@ __global__ void __launch_bounds__(FUSED_THREADS, (RECIP ? MVR_FWD_MINBLOCKS : MV
 // of its `per` chunks of 256 target points (in order, deterministic) into a list in shared memory, every thread then
 // searches its entries of the list, and sums over its own mutual pairs afterwards (phase B needs no barrier: a thread
 // revisits exactly the entries it searched, so a warp that is done does not wait for the slowest one of the block).
-#ifndef MVR_REV_MAX_CHUNKS
-#define MVR_REV_MAX_CHUNKS 4
-#endif
-constexpr int REV_MAX_CHUNKS = MVR_REV_MAX_CHUNKS;
+constexpr int REV_MAX_CHUNKS = 4;   // the most fused_rev_chunks hands out
 template <int EST>
-__global__ void __launch_bounds__(FUSED_THREADS, MVR_REV_MINBLOCKS * (256 / FUSED_THREADS)) k_icp_reverse(const __grid_constant__ RevBatch batch) {
+__global__ void __launch_bounds__(FUSED_THREADS, REV_MINBLOCKS * (256 / FUSED_THREADS)) k_icp_reverse(const __grid_constant__ RevBatch batch) {
   __shared__ RevArgs s_args;
   static_assert(sizeof(RevArgs) % 4 == 0 && sizeof(RevArgs) / 4 <= FUSED_THREADS, "argument block");
   if (threadIdx.x < sizeof(RevArgs) / 4) ((uint32_t*)&s_args)[threadIdx.x] = ((const uint32_t*)&batch.a[blockIdx.y])[threadIdx.x];
@@ -571,7 +554,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, MVR_REV_MINBLOCKS * (256 / FUSE
     const float dev = dev0 + 1.0e-6f * fmaxf(fabsf(ux), fmaxf(fabsf(uy), fabsf(uz)));
     // a chooser sits at exactly this distance: the lexicographic minimum (d2, index) over all source points is found
     NnBest b{__uint_as_float((uint32_t)s_p[k]), 0x7fffffff, -1};
-    pg_search<MVR_PG_UNROLL>(a.gs, a.sstart, a.cur, a.n_valid, t.x, t.y, t.z, ux, uy, uz, dev, stretch, MVR_INF, b, seg);
+    pg_search<PG_UNROLL>(a.gs, a.sstart, a.cur, a.n_valid, t.x, t.y, t.z, ux, uy, uz, dev, stretch, MVR_INF, b, seg);
     if (b.pos < 0) ++missed;
     const int mutual = (b.pos >= 0 && __ldg(a.corr_p + b.pos) == j) ? b.pos : -1;   // or the nearest source point chose another target
     s_p[k] = mutual;
@@ -594,7 +577,6 @@ __global__ void __launch_bounds__(FUSED_THREADS, MVR_REV_MINBLOCKS * (256 / FUSE
   }
   reduce_and_finish<NV, EST == EST_SYM>(v, a.partials, st, a.log, a.grid);
 }
-#endif   // MVR_TS_TILE
 
 // (Tried in round 2 and dropped, profiles/r02_dynamic_items_ab.log: resident blocks drawing their chunks from a counter instead of
 // one block per chunk -- 12 % slower with 24 pairs per launch, no gain with 3.)
@@ -603,18 +585,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, MVR_REV_MINBLOCKS * (256 / FUSE
 // one 200k pair alone): 2 chunks 25.3 ms / 2.06 ms, 3 chunks 24.1 / 2.08, 4 chunks 24.0 / 2.23 -- three chunks, four once
 // a cloud fills the GPU on its own.  A pure function of the cloud size, so that the block partition, and with it the
 // order of the sums, does not depend on what else runs in the batch.
-int fused_rev_chunks(int items) {
-#ifdef MVR_REV_CHUNKS
-  return MVR_REV_CHUNKS;
-#else
-#ifdef MVR_TS_TILE
-  (void)items;
-  return 2;   // about half of the target points are chosen: two chunks fill one tile of 256 searches
-#else
-  return items >= 400000 ? 4 : 3;
-#endif
-#endif
-}
+int fused_rev_chunks(int items) { return items >= 400000 ? 4 : 3; }
 int fused_grid_rev(int items) {
   const int chunks = (items + FUSED_THREADS - 1) / FUSED_THREADS;
   const int per = fused_rev_chunks(items);
@@ -627,21 +598,8 @@ int fused_grid(int items) {
   return blocks < 1 ? 1 : (blocks > FUSED_MAX_BLOCKS ? FUSED_MAX_BLOCKS : blocks);
 }
 
-#ifdef MVR_SMEM_CARVEOUT
-static void set_carveout_once() {
-  static bool done = false;
-  if (done) return;
-  done = true;
-  cudaFuncSetAttribute(k_icp_forward<true, EST_P2P>, cudaFuncAttributePreferredSharedMemoryCarveout, MVR_SMEM_CARVEOUT);
-  cudaFuncSetAttribute(k_icp_reverse<EST_P2P>, cudaFuncAttributePreferredSharedMemoryCarveout, MVR_SMEM_CARVEOUT);
-}
-#else
-static void set_carveout_once() {}
-#endif
-
 cudaError_t launch_icp_forward(const FwdBatch& d_batch, int pairs, int max_grid, int first, bool reciprocal, int est, cudaStream_t s) {
   if (pairs <= 0 || pairs > FUSED_MAX_PAIRS) return pairs <= 0 ? cudaSuccess : cudaErrorInvalidValue;
-  set_carveout_once();
   const dim3 grid((unsigned)max_grid, (unsigned)pairs);
   if (reciprocal) {
     // the reciprocal forward half accumulates nothing: one instantiation serves every estimator but the symmetric one, whose
@@ -683,7 +641,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, 4) k_pair_nn(const float4* __re
   if (i >= n) return;
   const float4 p = __ldg(q + i);
   NnBest b{MVR_INF, 0x7fffffff, -1};
-  if (finite3(p)) pg_search<MVR_PG_UNROLL>(g, tstart, tgt, m_valid, p.x, p.y, p.z, p.x, p.y, p.z, 0.0f, 1.0f, MVR_INF, b, s_seg + threadIdx.x);
+  if (finite3(p)) pg_search<PG_UNROLL>(g, tstart, tgt, m_valid, p.x, p.y, p.z, p.x, p.y, p.z, 0.0f, 1.0f, MVR_INF, b, s_seg + threadIdx.x);
   const int o = BY_W ? __float_as_int(p.w) : i;
   out_idx[o] = b.pos >= 0 ? b.idx : -1;
   out_d2[o] = b.pos >= 0 ? b.d2 : MVR_INF;

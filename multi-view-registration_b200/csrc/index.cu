@@ -118,7 +118,7 @@ cudaError_t launch_bbox(const float4* pts, int n, uint32_t* out7, cudaStream_t s
 }
 
 // ---------------------------------------------------------------------------------------------
-// Morton keys (K1) and the fused per-iteration transform + keys (K7 + K1)
+// Morton keys (K1)
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_morton_keys(const float4* __restrict__ pts, int n, GridDev g,
                                                      uint32_t* __restrict__ keys, uint32_t* __restrict__ vals) {
@@ -126,22 +126,6 @@ __global__ void __launch_bounds__(256) k_morton_keys(const float4* __restrict__ 
   if (i >= n) return;
   keys[i] = point_key(__ldg(pts + i), g);
   vals[i] = (uint32_t)i;
-}
-
-__global__ void __launch_bounds__(256) k_transform_keys(float4* __restrict__ pts, int n, Mat4f M, GridDev g,
-                                                        uint32_t* __restrict__ keys, uint32_t* __restrict__ vals) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  float4 p = pts[i];
-  if (finite3(p)) { p = xform_pinned(M, p); pts[i] = p; }
-  if (keys) { keys[i] = point_key(p, g); vals[i] = (uint32_t)i; }
-}
-
-__global__ void __launch_bounds__(256) k_transform(const float4* __restrict__ in, float4* __restrict__ out, int n, Mat4f M) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  float4 p = __ldg(in + i);
-  out[i] = finite3(p) ? xform_pinned(M, p) : p;
 }
 
 // PointCloud::getTransformedPoints (mvr/src/point_cloud.cpp:290-303): p' = pose * p evaluated in double and
@@ -201,18 +185,6 @@ cudaError_t launch_apply_pose(const void* in, size_t stride, int n, const double
 cudaError_t launch_morton_keys(const float4* pts, int n, GridDev g, uint32_t* keys, uint32_t* vals, cudaStream_t s) {
   if (n <= 0) return cudaSuccess;
   k_morton_keys<<<(n + 255) / 256, 256, 0, s>>>(pts, n, g, keys, vals); count_launch();
-  return cudaGetLastError();
-}
-
-cudaError_t launch_transform_keys(float4* pts, int n, Mat4f M, GridDev g, uint32_t* keys, uint32_t* vals, cudaStream_t s) {
-  if (n <= 0) return cudaSuccess;
-  k_transform_keys<<<(n + 255) / 256, 256, 0, s>>>(pts, n, M, g, keys, vals); count_launch();
-  return cudaGetLastError();
-}
-
-cudaError_t launch_transform(const float4* in, float4* out, int n, Mat4f M, cudaStream_t s) {
-  if (n <= 0) return cudaSuccess;
-  k_transform<<<(n + 255) / 256, 256, 0, s>>>(in, out, n, M); count_launch();
   return cudaGetLastError();
 }
 

@@ -28,9 +28,6 @@ cudaError_t launch_bbox_batch(const BboxBatch& batch, int count, uint32_t* out7,
 cudaError_t launch_apply_pose(const void* in, size_t stride, int n, const double* M16, float4* out, cudaStream_t s);
 
 cudaError_t launch_morton_keys(const float4* pts, int n, GridDev g, uint32_t* keys, uint32_t* vals, cudaStream_t s);
-// In-place pinned transform of pts followed by key generation (ICP's per-iteration transformCloud).
-cudaError_t launch_transform_keys(float4* pts, int n, Mat4f M, GridDev g, uint32_t* keys, uint32_t* vals, cudaStream_t s);
-cudaError_t launch_transform(const float4* in, float4* out, int n, Mat4f M, cudaStream_t s);
 
 struct SortScratch {
   uint32_t* keys_alt;   // n
@@ -46,19 +43,6 @@ cudaError_t launch_radix_sort(uint32_t* keys, uint32_t* vals, int n, int key_bit
 cudaError_t launch_gather_sorted(const float4* pts, const uint32_t* perm, int n, float4* sorted, cudaStream_t s);
 // start[c] = first sorted position with key >= c, for c in [0, 1 << 3*bits].
 cudaError_t launch_cell_table(const uint32_t* sorted_keys, int n, int bits, uint32_t* start, cudaStream_t s);
-
-// ---- bin.cu --------------------------------------------------------------------------------
-// Counting sort of a (moving) cloud by grid cell: see bin.cu.  counters has cells+1 entries (the last
-// one collects non-finite points) and must be zero on entry (k_scan_cells re-zeroes it); start gets
-// cells+2 entries.  d_delta (nullable): device float[16] applied in place before binning.  d_done
-// (nullable): device flag, non-zero turns the launch into a no-op.
-cudaError_t launch_transform_bin(float4* pts, int n, const float* d_delta, const int* d_done, GridDev g, uint32_t* keys,
-                                 uint32_t* rank, uint32_t* counters, cudaStream_t s);
-int scan_num_tiles(size_t len);
-cudaError_t launch_scan_cells(uint32_t* counters, uint32_t* start, size_t len, unsigned long long* tile_state, uint32_t epoch,
-                              const int* d_done, cudaStream_t s);
-cudaError_t launch_bin_scatter(const float4* pts, int n, const uint32_t* keys, const uint32_t* rank, const uint32_t* start,
-                               const int* d_done, float4* sorted, cudaStream_t s);
 
 // ---- icp.cu --------------------------------------------------------------------------------
 enum { REDUCE_P2P_VALS = 18, REDUCE_P2L_VALS = 30, REDUCE_MOM_VALS = 30, REDUCE_MAX_VALS = 32, REDUCE_BLOCKS = 592, ICP_MAX_LOG = 1024 };
@@ -86,8 +70,7 @@ struct IcpState {
   int max_iter, fixed, min_corr, p2l, recip, n_src;   // p2l: estimator of the solve, 0 point-to-point, 1 point-to-plane, 2 symmetric
   unsigned int ticket;    // blocks of the running reduction that have finished
   long long dbg[8];       // diagnostics: [0] clock cycles spent in the serial solve, [1] solves, [2] reciprocal searches that lost their chooser (must be 0),
-                          // [3] forward queries answered by the per-thread fallback, [4] forward rounds whose tile did not fit,
-                          // [5] / [6] the same for the reciprocal half, [7] forward queries settled by the gate mask
+                          // [3] (staged copy only) the pair's crowded word, see InitJob, [4..7] unused
   // frame bookkeeping of the static source index (pair_index.cu / pair_search.cuh)
   double cum[16];         // increments applied since the source was binned, incl. the pending `delta`, column-major
   double cinv[12];        // its affine inverse, rows {A^-1 | -A^-1 b}
@@ -101,14 +84,11 @@ struct IcpState {
 };
 
 // ---- fused iteration (icp.cu) + per-align index (pair_index.cu) ---------------------------------
-#ifndef MVR_FUSED_THREADS
-#define MVR_FUSED_THREADS 256
-#endif
 // grid = min(ceil(items / FUSED_THREADS), FUSED_MAX_BLOCKS): a pure function of the cloud size
-enum { FUSED_THREADS = MVR_FUSED_THREADS, FUSED_WARPS = FUSED_THREADS / 32, FUSED_MAX_BLOCKS = 148 * 8 * (256 / FUSED_THREADS) };
+enum { FUSED_THREADS = 256, FUSED_WARPS = FUSED_THREADS / 32, FUSED_MAX_BLOCKS = 148 * 8 * (256 / FUSED_THREADS) };
 
 // Deterministic counting sort of a cloud by row-major cell (pair_index.cu): count (keys + arrival ranks; counters
-// has cells + 1 zeroed entries, the last one collects non-finite points), scan (bin.cu), scatter into tmp in arrival
+// has cells + 1 zeroed entries, the last one collects non-finite points), scan, scatter into tmp in arrival
 // order, rerank into ascending original index inside every cell.  A BuildJob describes one build; one launch per
 // phase serves every job of a BuildBatch (blockIdx.y = job).
 struct BuildJob {
@@ -133,7 +113,7 @@ struct BuildJob {
 enum { BUILD_MAX_JOBS = 48 };
 struct BuildBatch { BuildJob j[BUILD_MAX_JOBS]; };
 cudaError_t launch_pair_builds(const BuildBatch& batch, int count, cudaStream_t s);
-cudaError_t launch_scan_cells_batch(const BuildBatch& batch, int count, int max_tiles, cudaStream_t s);
+int scan_num_tiles(size_t len);   // tiles of the scan over a table of len counters
 // Gate mask of an index (pair_index.cu): occ and mask hold ny * nz * wstride words, wstride = ceil(nx / 32); D / Dx = dilation in
 // y-z / x cells.
 cudaError_t launch_gate_mask(const uint32_t* start, PairGrid g, int wstride, int D, int Dx, uint32_t* occ, uint32_t* mask, cudaStream_t s);

@@ -16,22 +16,42 @@
 //     evaluated on the CURRENT coordinates, so results are bit-identical to a search over a freshly
 //     built index.  What the stale cells cost is a slack on every geometric bound, see below.
 //
-// Exactness.  Let a candidate k have pinned float d2(t, cur_k) <= lim; then |t - cur_k| <= rho with
-// rho = sqrt(lim) (1 + 2^-22).  With C x = A x + b the accumulated increment since binning and
-// dev >= |cur_k - C s0_k| for every k (MEASURED by the forward kernel in the same iteration):
+// Exactness, first for points that have not moved (dev = 0, stretch = 1: the target of the forward half,
+// every index but the moving source).  grid_t() rounds with |error| <= 2^-23 |t| per point;
+// margin (cells) = MVR_CELL_MARGIN + 1e-6 |t| absorbs that on both the query and the indexed point.  A
+// point whose pinned float d2 is <= lim has |p_a - q_a| <= sqrt(lim) (1 + 2^-22) on every axis, hence its
+// cell coordinate lies in [floor(t_a - rc), floor(t_a + rc)] with rc = sqrt(lim) inv_cell (1 + 1e-6) +
+// margin: the box of rows walked below cannot miss it.  Lower bounds of rows and cells shrink the
+// geometric gap by margin, use cell_lo (a float strictly below the true cell edge) and a relative 1e-6
+// (MVR_REL_SHRINK), so lb is a true lower bound on the float d2 of every point filed there; a row or cell
+// is skipped only when lb exceeds the running limit (strictly), so equal-distance ties with a lower index
+// are never cut off.
+// Points that moved rigidly: let a candidate k have pinned float d2(t, cur_k) <= lim; then |t - cur_k| <= rho
+// with rho = sqrt(lim) (1 + 2^-22).  With C x = A x + b the accumulated increment since binning and
+// dev >= |cur_k - C s0_k| for every k (bounded analytically by the solve, icp.cu icp_advance_frame):
 //     u - s0_k = A^-1 (t - C s0_k)   =>   |u - s0_k| <= stretch (rho + dev),   stretch >= ||A^-1||_2.
 // Hence s0_k's cell lies inside the box of radius rc = (sqrt(lim) stretch inv_cell)(1 + 1e-6) + margin
-// around u's scaled coordinate, where margin (cells) = MVR_CELL_MARGIN + 1e-6 |t| (rounding of grid_t on
-// both sides, as in nn_search.cuh) + dev stretch inv_cell.  Conversely a point whose cell is gamma away
-// from u (per-axis gaps already shrunk by margin) has |t - cur_k| >= |gamma| cell / stretch, so a row or
-// cell is skipped only when that lower bound exceeds the running limit (strictly): equal-distance ties
-// with a lower index are never cut off.  With dev = 0, stretch = 1 (forward half: the target does not
-// move) this reduces to the bounds of nn_search.cuh.  Boundary cells are unbounded outwards: points and
-// queries outside the grid are filed in / start from the clamped cell.
+// around u's scaled coordinate, where margin grows by dev stretch inv_cell.  Conversely a point whose cell
+// is gamma away from u (per-axis gaps already shrunk by margin) has |t - cur_k| >= |gamma| cell / stretch,
+// so the same strict test holds with cell_lo / stretch for the cell edge.  Boundary cells are unbounded
+// outwards (cell_gap): points and queries outside the grid are filed in / start from the clamped cell.
 #pragma once
-#include "nn_search.cuh"
+#include "common.cuh"
 
 namespace mvr {
+
+struct NnBest {
+  float d2;
+  int idx;   // original index of the best point, INT_MAX if none
+  int pos;   // its position in the sorted array (-1 for a seed)
+};
+
+// Gap (cells, >= 0) between scaled coordinate t and the slab of cell c, boundary cells unbounded outwards.
+__device__ __forceinline__ float cell_gap(float t, int c, int G) {
+  float lo = (c > 0) ? (float)c - t : 0.0f;
+  float hi = (c < G - 1) ? t - (float)(c + 1) : 0.0f;
+  return fmaxf(fmaxf(lo, hi), 0.0f);
+}
 
 __device__ __forceinline__ int pg_cell(float t, int n) { return (int)fminf(fmaxf(floorf(t), 0.0f), (float)(n - 1)); }
 
@@ -62,10 +82,7 @@ __device__ __forceinline__ void pg_scan(const float4* __restrict__ pts, uint32_t
 }
 
 // Segment list of one thread in shared memory: slot j of thread t lives at seg[j * PG_STRIDE + t] (bank = t).
-#ifndef MVR_PG_SEGS
-#define MVR_PG_SEGS 8
-#endif
-constexpr int PG_SEGS = MVR_PG_SEGS;   // row segments collected before a flat scan
+constexpr int PG_SEGS = 8;   // row segments collected before a flat scan
 constexpr int PG_STRIDE = FUSED_THREADS;
 
 // Flat scan of the thread's collected segments: ONE loop over all candidates of all rows, UNROLL independent loads per
