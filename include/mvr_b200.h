@@ -253,6 +253,19 @@ int mvr_estimate_normals(mvr_ctx* ctx, int which, int k, const float viewpoint[3
  * no target; an empty target is MVR_OK with nothing to do.  No context may appear twice; k in 3..32. */
 int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const float* viewpoints, float* const* out_nxyzc,
                                int* statuses);
+/* Score n_candidates rigid transforms of each context's source against its target (device of ctxs[0]).
+ * candidates: count x n_candidates x float[16] column-major; costs: count x n_candidates; inliers nullable.
+ * samples: 1..65536; n_candidates: 1..1024.  statuses[k]: MVR_ERR_NO_INPUT without source/target;
+ * an empty source or target scores samples x 2^24 / 0 (no error).
+ * The samples are the finite source points of original index i % stride == 0, stride = max(1, ceil(n / samples)), the same for
+ * every candidate.  Each is moved by the candidate's float transform (the one an align applies to its guess) and its exact
+ * nearest target point within the gate max_dist is looked up; it costs floor(d2 * 2^24 / g), at most 2^24, when that neighbour
+ * passes the align's gate test (d2 <= max_dist^2, g = the gate as a float rounded up), 2^24 otherwise.  costs = the sum over the
+ * samples, inliers = the samples within the gate: integers, exact whatever the GPU.  Each context's target index is the one an
+ * align with the same max_dist uses: that align does not build it again, and a second call on unchanged targets builds none.
+ * No context may appear twice; the call returns when the results are on the host. */
+int mvr_score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
+                            uint64_t* costs, int32_t* inliers, int* statuses);
 
 /* -- pose application: PointCloud::getTransformedPoints (mvr/src/point_cloud.cpp:290-303) ------------
  * out[i] = {float(pose * p_i), 1}: the multiply runs in double (osg::Matrix is double) and is narrowed to
@@ -345,6 +358,25 @@ int mvr_pairwise_align(mvr_registrator* r, const mvr_view* source, const mvr_vie
  * gather).  reports: one per pair (ring: V entries indexed by pair; accumulate: V-1 entries, views 1..V-1). */
 int mvr_register_turntable(mvr_registrator* r, const mvr_view* views, int n_views, const mvr_turntable_params* prm,
                            float* poses, mvr_pair_report* reports);
+/* Ring mode only (the other modes ignore it): search turns about the turntable axis around each pair's initial guess before the
+ * first align, for tables that step unevenly, slip or are turned by hand.  The candidates of pair p (target view T = p, source
+ * view S = p + 1) are H_j = inv(T.pose) R(delta_j) S.pose, R = the turntable rotation (mvr_turntable_rotation), j = -J..J;
+ * all pairs are scored by one mvr_score_guesses_batch with icp.max_correspondence_distance and each pair starts from its
+ * lowest-cost H_j (ties: the smallest |j|, then the smaller j; H_0 is the guess without the search).  The choice depends only
+ * on the pair's views, their poses and this setting: pair poses stay the same whatever the streams, grouping, pair ranges or
+ * GPU count.  Off by default. */
+typedef struct {
+  double range;  /* radians; candidate turns about the axis span [-range, +range] around each pair's guess; <= 0: off */
+  double step;   /* radians, > 0; candidates delta_j = j * step, j = -J..J, J = lround(range / step), 2J + 1 <= 1024 */
+  int samples;   /* source points scored per candidate (0: 4096) */
+} mvr_angle_search;
+void mvr_angle_search_default(mvr_angle_search* s);   /* 15 degrees, 1 degree, 4096 */
+int mvr_registrator_set_angle_search(mvr_registrator* r, const mvr_angle_search* s);   /* NULL or range <= 0: off */
+/* One record per pair of the last ring registration with the search on: choice = j, angle = delta_j, cost / inliers of H_j,
+ * samples = the source points scored, guess_cost / guess_inliers = those of H_0. */
+typedef struct { int pair; int choice; double angle; uint64_t cost; int inliers; int samples;
+                 uint64_t guess_cost; int guess_inliers; } mvr_angle_pick;
+int mvr_registrator_get_angle_search(mvr_registrator* r, mvr_angle_pick* out, int max_records, int* count);   /* out NULL: count only */
 /* -- the same entry point over several GPUs of one node ----------------------------------------------------------
  * The reference is one process (its registration runs on one pool thread, mvr/src/registrator.cpp:606, 696); what shards
  * is the ring of neighbour pairs (the edges of :640-651 / :482-487).  One call, inside: one host thread per GPU aligns a
@@ -380,6 +412,9 @@ int mvr_multi_upload(mvr_multi* m, const mvr_view* views, int n_views);
  * (nullable): per GPU, the device time of its part including the exchange (CUDA events). */
 int mvr_register_turntable_multi(mvr_multi* m, const mvr_view* views, int n_views, const mvr_turntable_params* prm, int use_resident,
                                  float* poses, mvr_pair_report* reports, mvr_pair_record* records, double* device_ms);
+/* mvr_registrator_set_angle_search on every rank; the records of the last call, in pair order (out NULL: count only). */
+int mvr_multi_set_angle_search(mvr_multi* m, const mvr_angle_search* s);
+int mvr_multi_get_angle_search(mvr_multi* m, mvr_angle_pick* out, int max_records, int* count);
 
 /* Registrator::computeError (mvr/src/registrator.cpp:466-515): reciprocal correspondences (gate max_distance) between
  * neighbouring registered views (i, i + 1) and (V - 1, 0), each view posed by its init_pose first (getTransformedPoints).

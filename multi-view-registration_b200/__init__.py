@@ -110,6 +110,21 @@ class PairMoments(C.Structure):
                     sba=np.array(self.sba[:]).reshape(3, 3), saa=np.array(self.saa[:]), sbb=np.array(self.sbb[:]), d2=self.d2)
 
 
+class AngleSearch(C.Structure):
+    """mvr_angle_search: turns about the turntable axis the ring driver scores around each pair's guess (range <= 0: off)."""
+    _fields_ = [("range", C.c_double), ("step", C.c_double), ("samples", C.c_int)]
+
+
+class AnglePick(C.Structure):
+    """mvr_angle_pick: the turn a ring pair started from (choice = j, angle = j * step) and its score against the guess's (j = 0)."""
+    _fields_ = [("pair", C.c_int), ("choice", C.c_int), ("angle", C.c_double), ("cost", C.c_uint64), ("inliers", C.c_int),
+                ("samples", C.c_int), ("guess_cost", C.c_uint64), ("guess_inliers", C.c_int)]
+
+    def as_dict(self):
+        return dict(pair=self.pair, choice=self.choice, angle=self.angle, cost=int(self.cost), inliers=self.inliers, samples=self.samples,
+                    guess_cost=int(self.guess_cost), guess_inliers=self.guess_inliers)
+
+
 class ViewDesc(C.Structure):
     _fields_ = [("xyzw", C.c_void_p), ("n", C.c_size_t), ("on_device", C.c_int), ("init_pose", C.POINTER(C.c_double))]
 
@@ -206,6 +221,13 @@ def lib():
     L.mvr_estimate_normals.argtypes = [vp, C.c_int, C.c_int, fp, fp, ip]
     L.mvr_estimate_normals_batch.argtypes = [C.POINTER(vp), C.c_int, C.c_int, fp, C.POINTER(fp), ip]
     dp = C.POINTER(C.c_double)
+    L.mvr_score_guesses_batch.argtypes = [C.POINTER(vp), C.c_int, fp, C.c_int, C.c_double, C.c_int, C.POINTER(C.c_uint64), ip, ip]
+    L.mvr_angle_search_default.argtypes = [C.POINTER(AngleSearch)]
+    L.mvr_angle_search_default.restype = None
+    L.mvr_registrator_set_angle_search.argtypes = [vp, C.POINTER(AngleSearch)]
+    L.mvr_registrator_get_angle_search.argtypes = [vp, C.POINTER(AnglePick), C.c_int, C.POINTER(C.c_int)]
+    L.mvr_multi_set_angle_search.argtypes = [vp, C.POINTER(AngleSearch)]
+    L.mvr_multi_get_angle_search.argtypes = [vp, C.POINTER(AnglePick), C.c_int, C.POINTER(C.c_int)]
     L.mvr_apply_pose.argtypes = [vp, vp, C.c_size_t, C.c_size_t, dp, fp]
     L.mvr_apply_pose_device.argtypes = [vp, vp, C.c_size_t, C.c_size_t, dp, vp]
     L.mvr_copy_aligned_device.argtypes = [vp, vp]
@@ -713,6 +735,48 @@ def estimate_normals_batch(contexts, k, viewpoints=None, want=False):
     return outs
 
 
+def score_guesses_batch(contexts, candidates, max_dist, samples=4096):
+    """mvr_score_guesses_batch: candidates = len(contexts) x n_candidates 4x4 transforms (source -> target frame).  Returns
+    (costs len(contexts) x n_candidates uint64, inliers the same shape int32, statuses int32 per context); raises on a failure
+    of the batch itself (a context without input only sets its status)."""
+    n = len(contexts)
+    M = np.asarray(candidates, dtype=np.float32)
+    if M.ndim != 4 or M.shape[0] != n or M.shape[2:] != (4, 4):
+        raise ValueError("candidates must be len(contexts) x n_candidates x 4 x 4")
+    nc = M.shape[1]
+    flat = np.ascontiguousarray(M.transpose(0, 1, 3, 2)).reshape(-1)   # column-major per candidate
+    hs = (C.c_void_p * max(n, 1))(*[c._h for c in contexts])
+    costs = np.zeros((max(n, 1), nc), dtype=np.uint64)
+    inl = np.zeros((max(n, 1), nc), dtype=np.int32)
+    st = np.zeros(max(n, 1), dtype=np.int32)
+    rc = lib().mvr_score_guesses_batch(hs, n, _fp(flat) if n else None, int(nc), float(max_dist), int(samples),
+                                       costs.ctypes.data_as(C.POINTER(C.c_uint64)), _ip(inl), _ip(st))
+    if rc != OK:
+        raise MvrError(rc, contexts[0].last_error() if n else lib().mvr_status_string(rc).decode())
+    return costs[:n], inl[:n], st[:n]
+
+
+def angle_search_default():
+    s = AngleSearch()
+    lib().mvr_angle_search_default(C.byref(s))
+    return s
+
+
+def _angle_search(range_, step, samples):
+    if range_ is None or range_ <= 0:
+        return None
+    d = angle_search_default()
+    return AngleSearch(float(range_), d.step if step is None else float(step), int(samples))
+
+
+def _picks(getter, h):
+    n = C.c_int(0)
+    getter(h, None, 0, C.byref(n))
+    arr = (AnglePick * max(n.value, 1))()
+    getter(h, arr, n.value, C.byref(n))
+    return [arr[k].as_dict() for k in range(n.value)]
+
+
 def pair_moments_transform(m, pose, new_origin=None):
     """Moments of the pairs after the rigid map p -> pose * p (4x4), about new_origin (default pose * origin)."""
     P = np.ascontiguousarray(np.asarray(pose, dtype=np.float64).T).reshape(16)
@@ -818,6 +882,18 @@ class Registrator:
         return dict(status=rc, final=pose_to_numpy(fin), iterations=rep.iterations, n_corr=rep.n_correspondences, mse=rep.mse,
                     gpu_ms=rep.gpu_ms, nn_queries=int(rep.nn_queries))
 
+    def set_angle_search(self, range=None, step=None, samples=0):
+        """Ring mode: score turns about the axis, j * step for |j| <= lround(range / step) (radians; step None: 1 degree), around
+        every pair's guess and start each pair from the best (mvr_registrator_set_angle_search).  range None or <= 0: off."""
+        s = _angle_search(range, step, samples)
+        rc = lib().mvr_registrator_set_angle_search(self._h, C.byref(s) if s is not None else None)
+        if rc != OK:
+            raise MvrError(rc, (lib().mvr_registrator_last_error(self._h) or b"").decode())
+
+    def angle_search_log(self):
+        """One dict per pair of the last ring registration with the search on (AnglePick fields)."""
+        return _picks(lib().mvr_registrator_get_angle_search, self._h)
+
     def fitness_log(self):
         """[(view, repeat, getFitnessScore())] of the last accumulative registration (the reference's fitness_scores.txt)."""
         n = C.c_int(0)
@@ -898,6 +974,15 @@ class MultiRegistrator:
     def contexts(self, rank):
         """The (borrowed) Contexts of one rank."""
         return [Context(_borrowed=lib().mvr_multi_context(self._h, int(rank), k)) for k in range(int(lib().mvr_multi_contexts(self._h, int(rank))))]
+
+    def set_angle_search(self, range=None, step=None, samples=0):
+        """Registrator.set_angle_search on every rank."""
+        s = _angle_search(range, step, samples)
+        self._ck(lib().mvr_multi_set_angle_search(self._h, C.byref(s) if s is not None else None))
+
+    def angle_search_log(self):
+        """The records of every rank's pairs, in pair order."""
+        return _picks(lib().mvr_multi_get_angle_search, self._h)
 
     def upload(self, views, init_poses=None):
         arr, keep = Registrator._views(views, init_poses)

@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 HOST = os.path.join(HERE, "host")
 LIB = os.path.join(HERE, "libmvr_b200.so")
 
-CU_SOURCES = ["index.cu", "pair_index.cu", "cell_nn.cu", "icp.cu", "normals.cu", "denoise.cu", "api.cu"]
+CU_SOURCES = ["index.cu", "pair_index.cu", "cell_nn.cu", "icp.cu", "normals.cu", "denoise.cu", "score.cu", "api.cu"]
 HOST_SOURCES = ["registrator.cpp", "lum.cpp", "capi.cpp", "multi.cpp"]
 
 NVCC_FLAGS = [

@@ -34,6 +34,8 @@ unsigned long long launch_count() { return g_launches.load(std::memory_order_rel
 // host/registrator.h
 int estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int count, int k, const float* viewpoints, float* const* out_nxyzc,
                            int* statuses);
+int score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
+                        uint64_t* costs, int32_t* inliers, int* statuses, int32_t* scored);
 }  // namespace mvr
 
 namespace {
@@ -126,6 +128,9 @@ struct mvr_ctx {
   int stage_cap = 0;
   DevBuf bbox_dev;               // 7 words per cloud of a batched mvr_set_clouds_device
   uint32_t* h_bbox = nullptr;    // pinned, BBOX_MAX_JOBS * 7 words
+  DevBuf score_dev;              // mvr_score_guesses_batch led by this context: candidate table, then the sums
+  unsigned char* h_score = nullptr;   // pinned staging of the same layout, score_cap bytes
+  size_t score_cap = 0;
   int log_pending = 0;           // records of the device log not fetched yet (mvr_icp_get_iterations fetches them)
   bool out_pending = false;      // out_cloud has not been computed yet (materialize_out)
   DevBuf crowded;                        // one word: population of the most crowded cell an index build could not rank (0: none)
@@ -637,9 +642,10 @@ int mvr_ctx_destroy(mvr_ctx* ctx) {
   ctx->tgt.release(); ctx->src.release(); ctx->normals.release(); ctx->snormals.release(); ctx->nsrc.release();
   ctx->pt.release(); ctx->ps.release(); ctx->nt.release(); ctx->nq.release();
   for (auto& b : ctx->bs) { b.keys.release(); b.vals.release(); b.moved.release(); b.count.release(); b.tiles.release(); }
-  ctx->stage_dev.release(); ctx->bbox_dev.release();
+  ctx->stage_dev.release(); ctx->bbox_dev.release(); ctx->score_dev.release();
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_bbox) cudaFreeHost(ctx->h_bbox);
+  if (ctx->h_score) cudaFreeHost(ctx->h_score);
   DevBuf* bufs[] = {&ctx->corr_p, &ctx->rmin, &ctx->rnn, &ctx->corr_j, &ctx->corr_d2, &ctx->partials, &ctx->sums, &ctx->out_cloud, &ctx->qtmp,
                     &ctx->itmp, &ctx->ftmp, &ctx->scratch, &ctx->misc, &ctx->state, &ctx->log, &ctx->crowded};
   for (DevBuf* b : bufs) b->release();
@@ -1781,10 +1787,122 @@ int mvr::estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int coun
   return rc;
 }
 
+// Declared in host/registrator.h: mvr_score_guesses_batch, plus scored[k] (nullable) = the finite samples of context k (`samples`
+// for an empty source or target).  Every context's target index is the one its align with the same max_dist builds (the
+// align's cell edge and grid, slot 0 of its build scratch): built here only when the context does not hold it yet, so the
+// align that follows finds it valid.  Like estimate_normals_batch, the work runs on the LEAD's stream after the work queued on
+// every context's stream; the call returns when the sums are on the host.
+int mvr::score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
+                             uint64_t* costs, int32_t* inliers, int* statuses, int32_t* scored) {
+  if (count < 0 || (count && (!ctxs || !candidates || !costs || !statuses))) return MVR_ERR_BAD_ARG;
+  if (count == 0) return MVR_OK;
+  for (int k = 0; k < count; ++k) {
+    if (!ctxs[k]) return MVR_ERR_BAD_ARG;
+    for (int j = 0; j < k; ++j) if (ctxs[j] == ctxs[k]) return fail(ctxs[0], MVR_ERR_BAD_ARG, "a context appears twice in the batch");
+    if (ctxs[k]->device != ctxs[0]->device) return fail(ctxs[0], MVR_ERR_BAD_ARG, "the contexts of a batch must share a device");
+  }
+  mvr_ctx* ctx = ctxs[0];   // the lead: CK() reports into it, its stream runs the batch, its profile records the launches
+  if (n_candidates < 1 || n_candidates > (int)SCORE_MAX_CANDIDATES) return fail(ctx, MVR_ERR_BAD_ARG, "n_candidates must be in 1..1024");
+  if (samples < 1 || samples > 65536) return fail(ctx, MVR_ERR_BAD_ARG, "samples must be in 1..65536");
+  if (!(max_dist >= 0)) return fail(ctx, MVR_ERR_BAD_ARG, "max_dist must be >= 0");
+  cudaSetDevice(ctx->device);
+  const cudaStream_t S = ctx->stream;
+  const size_t nc = (size_t)n_candidates, cells_all = (size_t)count * nc;
+  const size_t off_cost = cells_all * sizeof(Mat4f), off_in = off_cost + cells_all * sizeof(uint64_t), off_sc = off_in + cells_all * sizeof(uint32_t);
+  const size_t bytes = off_sc + (size_t)count * sizeof(uint32_t);
+  if (bytes > ctx->score_cap) {
+    if (ctx->h_score) cudaFreeHost(ctx->h_score);
+    ctx->h_score = nullptr; ctx->score_cap = 0;
+    CK(cudaMallocHost((void**)&ctx->h_score, bytes));
+    ctx->score_cap = bytes;
+  }
+  CK(ctx->score_dev.ensure(bytes));
+  unsigned char* d = ctx->score_dev.as<unsigned char>();
+  const float gate = gate_float(max_dist);
+  const float scale = (float)(16777216.0 / (double)gate);
+  std::vector<ScoreJob> jobs;
+  std::vector<int> job_ctx;
+  std::vector<BuildJob> builds;
+  for (int k = 0; k < count; ++k) {
+    mvr_ctx* m = ctxs[k];
+    for (size_t a = 0; a < nc; ++a) { costs[k * nc + a] = 0; if (inliers) inliers[k * nc + a] = 0; }
+    if (scored) scored[k] = 0;
+    if (m->tgt.gen == 0 || m->src.gen == 0) { statuses[k] = fail(m, MVR_ERR_NO_INPUT, "source/target not set"); continue; }
+    statuses[k] = MVR_OK;
+    if (m->src.n == 0 || m->tgt.n == 0) {   // nothing to score: every sample misses
+      for (size_t a = 0; a < nc; ++a) costs[k * nc + a] = (uint64_t)samples << 24;
+      if (scored) scored[k] = samples;
+      continue;
+    }
+    if (m != ctx && m->stream != S) {
+      CK(cudaEventRecord(m->ev_b, m->stream));
+      CK(cudaStreamWaitEvent(S, m->ev_b, 0));
+    }
+    uint32_t cells = 0;
+    const PairGrid gt = make_pair_grid(m->tgt.lo, m->tgt.hi, pair_cell_edge(m, m->tgt, max_dist), &cells, PG_XRATIO);
+    PairIndex& pt = m->pt;
+    if (!(pt.valid && pt.gen == m->tgt.gen && same_pair_grid(pt.g, gt))) {
+      BuildJob job;
+      pt.valid = false;
+      const int rc = plan_pair_index(m, pt, 0, m->tgt.pts, m->tgt.n, m->tgt.n_bad, nullptr, gt, cells, true, S, &job);
+      if (rc) { pt.valid = false; ctx->err = m->err; return rc; }
+      builds.push_back(job);
+      pt.gen = m->tgt.gen;
+    }
+    const int n = m->src.n, stride = std::max(1, (int)(((long long)n + samples - 1) / samples));
+    ScoreJob j{};
+    j.src = m->src.pts; j.stride = stride; j.slots = (n + stride - 1) / stride;
+    j.tgt = pt.sorted.as<float4>(); j.tstart = pt.start.as<uint32_t>(); j.g = pt.g; j.m_valid = pt.n_valid;
+    j.gate = gate; j.scale = scale; j.max2 = max_dist * max_dist;
+    j.cand = (const Mat4f*)d + k * nc;
+    j.cost = (unsigned long long*)(d + off_cost) + k * nc;
+    j.inliers = (uint32_t*)(d + off_in) + k * nc;
+    j.scored = (uint32_t*)(d + off_sc) + k;
+    jobs.push_back(j);
+    job_ctx.push_back(k);
+  }
+  if (jobs.empty()) return MVR_OK;
+  std::memcpy(ctx->h_score, candidates, off_cost);
+  CK(cudaMemcpyAsync(d, ctx->h_score, off_cost, cudaMemcpyHostToDevice, S));
+  CK(cudaMemsetAsync(d + off_cost, 0, bytes - off_cost, S));
+  int rc = run_pair_builds(ctx, builds.data(), (int)builds.size(), S);
+  if (rc) return rc;
+  for (size_t k0 = 0; k0 < jobs.size(); k0 += BUILD_MAX_JOBS) {
+    const int c = (int)std::min(jobs.size() - k0, (size_t)BUILD_MAX_JOBS);
+    ScoreBatch batch;
+    double queries = 0, tpts = 0;
+    for (int a = 0; a < c; ++a) {
+      batch.j[a] = jobs[k0 + a];
+      queries += (double)jobs[k0 + a].slots * (double)nc;
+      tpts += ctxs[job_ctx[k0 + a]]->tgt.n;
+    }
+    ProfScope ps(ctx, MVR_K_NN, 24.0 * queries + 16.0 * tpts, queries, 1, S);
+    CK(launch_score(batch, c, n_candidates, S));
+  }
+  CK(cudaMemcpyAsync(ctx->h_score + off_cost, d + off_cost, bytes - off_cost, cudaMemcpyDeviceToHost, S));
+  CK(cudaStreamSynchronize(S));
+  const uint64_t* hc = (const uint64_t*)(ctx->h_score + off_cost);
+  const uint32_t* hi = (const uint32_t*)(ctx->h_score + off_in);
+  const uint32_t* hs = (const uint32_t*)(ctx->h_score + off_sc);
+  for (int k : job_ctx) {
+    for (size_t a = 0; a < nc; ++a) {
+      costs[k * nc + a] = hc[k * nc + a];
+      if (inliers) inliers[k * nc + a] = (int32_t)hi[k * nc + a];
+    }
+    if (scored) scored[k] = (int32_t)hs[k];
+  }
+  return MVR_OK;
+}
+
 extern "C" {
 
 int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const float* viewpoints, float* const* out_nxyzc, int* statuses) {
   return mvr::estimate_normals_batch(ctxs, nullptr, count, k, viewpoints, out_nxyzc, statuses);
+}
+
+int mvr_score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
+                            uint64_t* costs, int32_t* inliers, int* statuses) {
+  return mvr::score_guesses_batch(ctxs, count, candidates, n_candidates, max_dist, samples, costs, inliers, statuses, nullptr);
 }
 
 }  // extern "C"

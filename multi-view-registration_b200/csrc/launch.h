@@ -251,4 +251,29 @@ struct NormalsBatch { NormalsJob j[BUILD_MAX_JOBS]; };
 // kNN(k) PCA normals of `count` (<= BUILD_MAX_JOBS) clouds in one launch, all with the same k.
 cudaError_t launch_normals(const NormalsBatch& batch, int count, int k, cudaStream_t s);
 
+// ---- score.cu -----------------------------------------------------------------------------
+// One context of mvr_score_guesses_batch: samples src[s * stride] (original order, s < slots; the finite ones count), nc candidate
+// transforms cand[0 .. nc), the target's per-align index (sorted / start / g, m_valid finite points) and the align's gate (max2
+// exact, gate = gate_float(max_dist), scale = float(2^24 / gate)).  Out (zeroed before the launch): cost[a] and inliers[a] per
+// candidate, *scored = the finite samples.
+struct ScoreJob {
+  const float4* src;
+  int slots, stride;
+  const float4* tgt;
+  const uint32_t* tstart;
+  PairGrid g;
+  int m_valid;
+  float gate, scale;
+  double max2;
+  const Mat4f* cand;
+  unsigned long long* cost;
+  uint32_t* inliers;
+  uint32_t* scored;
+};
+enum { SCORE_MAX_CANDIDATES = 1024 };
+struct ScoreBatch { ScoreJob j[BUILD_MAX_JOBS]; };
+static_assert(sizeof(ScoreBatch) + sizeof(int) <= 32764, "the batch's jobs must fit the kernel parameters");
+// `count` (<= BUILD_MAX_JOBS) contexts, all with nc (<= SCORE_MAX_CANDIDATES) candidates, in one launch (blockIdx.y = context).
+cudaError_t launch_score(const ScoreBatch& batch, int count, int nc, cudaStream_t s);
+
 }  // namespace mvr

@@ -152,6 +152,30 @@ int mvr_register_turntable(mvr_registrator* r, const mvr_view* views, int n_view
   return rc;
 }
 
+void mvr_angle_search_default(mvr_angle_search* s) {
+  if (!s) return;
+  s->range = 15.0 * M_PI / 180.0;
+  s->step = 1.0 * M_PI / 180.0;
+  s->samples = 4096;
+}
+
+int mvr_registrator_set_angle_search(mvr_registrator* r, const mvr_angle_search* s) {
+  if (!r) return MVR_ERR_BAD_ARG;
+  return r->reg->setAngleSearch(s);
+}
+
+int mvr_registrator_get_angle_search(mvr_registrator* r, mvr_angle_pick* out, int max_records, int* count) {
+  if (!r || !count) return MVR_ERR_BAD_ARG;
+  const std::vector<mvr_angle_pick>& log = r->reg->angleLog();
+  int n = (int)log.size();
+  if (out) {
+    n = std::min(n, std::max(max_records, 0));
+    if (n) std::memcpy(out, log.data(), (size_t)n * sizeof(mvr_angle_pick));
+  }
+  *count = n;
+  return MVR_OK;
+}
+
 int mvr_registrator_get_fitness_log(mvr_registrator* r, mvr_fitness_record* out, int max_records, int* count) {
   if (!r || !count) return MVR_ERR_BAD_ARG;
   const std::vector<mvr_fitness_record>& log = r->reg->fitnessLog();

@@ -350,4 +350,26 @@ int mvr_register_turntable_multi(mvr_multi* m, const mvr_view* views, int n_view
   return MVR_OK;
 }
 
+int mvr_multi_set_angle_search(mvr_multi* m, const mvr_angle_search* s) {
+  if (!m) return MVR_ERR_BAD_ARG;
+  for (size_t k = 0; k < m->ranks.size(); ++k) {
+    const int rc = m->ranks[k].reg->setAngleSearch(s);
+    if (rc) return fail(m, rc, m->ranks[k].reg->lastError());
+  }
+  return MVR_OK;
+}
+
+int mvr_multi_get_angle_search(mvr_multi* m, mvr_angle_pick* out, int max_records, int* count) {
+  if (!m || !count) return MVR_ERR_BAD_ARG;
+  std::vector<mvr_angle_pick> all;   // rank k holds the records of its block of pairs: rank order is pair order
+  for (const Rank& r : m->ranks) all.insert(all.end(), r.reg->angleLog().begin(), r.reg->angleLog().end());
+  int n = (int)all.size();
+  if (out) {
+    n = std::min(n, std::max(max_records, 0));
+    if (n) std::memcpy(out, all.data(), (size_t)n * sizeof(mvr_angle_pick));
+  }
+  *count = n;
+  return MVR_OK;
+}
+
 }  // extern "C"

@@ -381,8 +381,59 @@ int Registrator::automaticRegistration(std::vector<View>& views, int max_iterati
   return accumulate(views, order, icp, repeat_times, true, reports, true);
 }
 
+int Registrator::setAngleSearch(const mvr_angle_search* s) {
+  if (!s || !(s->range > 0)) { angle_ = mvr_angle_search{0.0, 0.0, 0}; return MVR_OK; }
+  if (!std::isfinite(s->range) || !(s->step > 0) || !std::isfinite(s->step)) return fail(MVR_ERR_BAD_ARG, "angle search: range and step must be finite, step > 0");
+  const double half = s->range / s->step;
+  if (!(half < 1024.0) || 2 * std::lround(half) + 1 > 1024) return fail(MVR_ERR_BAD_ARG, "angle search: 2 lround(range / step) + 1 must be <= 1024");
+  if (s->samples < 0 || s->samples > 65536) return fail(MVR_ERR_BAD_ARG, "angle search: samples must be in 0..65536 (0: 4096)");
+  angle_ = *s;
+  if (angle_.samples == 0) angle_.samples = 4096;
+  return MVR_OK;
+}
+
+int Registrator::searchAngles(const std::vector<View>& views, int p0, const std::vector<mvr_ctx*>& cs, double max_dist, std::vector<float>& guesses) {
+  const int V = (int)views.size(), P = (int)cs.size();
+  const int J = (int)std::lround(angle_.range / angle_.step), nc = 2 * J + 1;
+  // H_j = inv(T.pose) R(j step) S.pose in double, narrowed elementwise; H_0 is the guess itself (the same bits)
+  std::vector<float> cand((size_t)P * nc * 16);
+  for (int k = 0; k < P; ++k) {
+    const Matrix4d inv = inverseRigid(views[(size_t)(p0 + k)].pose);
+    const Matrix4d& sp = views[(size_t)((p0 + k + 1) % V)].pose;
+    for (int a = 0; a < nc; ++a) {
+      float* out = &cand[((size_t)k * nc + a) * 16];
+      if (a == J) { std::memcpy(out, &guesses[(size_t)k * 16], 16 * sizeof(float)); continue; }
+      const Matrix4f H = toFloat(multiply(inv, multiply(getRotationMatrix((a - J) * angle_.step), sp)));
+      std::memcpy(out, H.m, sizeof(H.m));
+    }
+  }
+  std::vector<uint64_t> cost((size_t)P * nc);
+  std::vector<int32_t> inl((size_t)P * nc), scored((size_t)P);
+  std::vector<int> st((size_t)P, 0);
+  int rc = score_guesses_batch(cs.data(), P, cand.data(), nc, max_dist, angle_.samples, cost.data(), inl.data(), st.data(), scored.data());
+  if (rc) return fail(rc, mvr_last_error(cs[0]));
+  for (int k = 0; k < P; ++k) {
+    if (st[(size_t)k]) return fail(st[(size_t)k], mvr_last_error(cs[(size_t)k]));
+    const size_t row = (size_t)k * nc;
+    int best = J;   // lowest cost; ties: the smallest |j|, then the smaller j (a flat cost keeps the turntable guess)
+    for (int a = 0; a < nc; ++a) {
+      const int j = a - J, jb = best - J;
+      if (cost[row + a] < cost[row + best] || (cost[row + a] == cost[row + best] && (std::abs(j) < std::abs(jb) || (std::abs(j) == std::abs(jb) && j < jb))))
+        best = a;
+    }
+    std::memcpy(&guesses[(size_t)k * 16], &cand[(row + best) * 16], 16 * sizeof(float));
+    mvr_angle_pick r{};
+    r.pair = p0 + k; r.choice = best - J; r.angle = (best - J) * angle_.step;
+    r.cost = cost[row + best]; r.inliers = inl[row + best]; r.samples = scored[(size_t)k];
+    r.guess_cost = cost[row + J]; r.guess_inliers = inl[row + J];
+    angle_log_.push_back(r);
+  }
+  return MVR_OK;
+}
+
 int Registrator::multiViewRegister(std::vector<View>& views, const mvr_turntable_params& prm, std::vector<mvr_pair_report>& reports) {
   if (!ok()) return fail(MVR_ERR_CUDA, "no GPU context");
+  angle_log_.clear();
   const int normal_k = prm.normal_k == 0 ? 16 : prm.normal_k;   // 0: a zero-filled struct gets the default
   if (normal_k < 3 || normal_k > 32) return fail(MVR_ERR_BAD_ARG, "normal_k must be in 3..32 (0: 16)");
   const int V = (int)views.size();
@@ -467,6 +518,8 @@ int Registrator::multiViewRegister(std::vector<View>& views, const mvr_turntable
       if ((rc = mvr_normals_share(cs[(size_t)k], MVR_CLOUD_SOURCE, cs[(size_t)j], MVR_CLOUD_TARGET))) return fail(rc, mvr_last_error(cs[(size_t)k]));
     }
   }
+  // opt-in: every pair starts from the best-scoring turn about the axis around its guess (mvr_registrator_set_angle_search)
+  if (angle_.range > 0 && (rc = searchAngles(views, p0, cs, prm.icp.max_correspondence_distance, guesses))) return rc;
   const double t_share = now();
   const int repeats = std::max(prm.repeat_times, 1);
   for (int r = 0; r < repeats; ++r) {

@@ -125,6 +125,10 @@ class Registrator {
   // North-star form: ring pairs [pair_begin, pair_end) aligned independently (concurrently over the streams),
   // then (when the whole ring was computed here) chained / relaxed into absolute poses.
   int multiViewRegister(std::vector<View>& views, const mvr_turntable_params& prm, std::vector<mvr_pair_report>& reports);
+  // mvr_registrator_set_angle_search: NULL or range <= 0 switches the search off
+  int setAngleSearch(const mvr_angle_search* s);
+  // one record per pair of the last ring registration with the search on (empty otherwise)
+  const std::vector<mvr_angle_pick>& angleLog() const { return angle_log_; }
 
  private:
   int accumulate(std::vector<View>& views, const std::vector<int>& order, const mvr_icp_params& icp, int repeat_times,
@@ -136,6 +140,10 @@ class Registrator {
   struct DeviceBuffer { void* p = nullptr; size_t cap = 0; bool ensure(size_t bytes); };
   std::vector<DeviceBuffer> view_cache_;   // device copies of host views, one upload per view and registration
   double objectRadius(int slot) const;   // half the largest extent of the target cloud last given to context `slot`
+  // the angle search of multiViewRegister: pair k of cs (target view p0 + k) starts from its best-scoring turn (guesses[k])
+  int searchAngles(const std::vector<View>& views, int p0, const std::vector<mvr_ctx*>& cs, double max_dist, std::vector<float>& guesses);
+  mvr_angle_search angle_{0.0, 0.0, 0};   // range <= 0: off
+  std::vector<mvr_angle_pick> angle_log_;
   int fail(int code, const std::string& msg) { std::lock_guard<std::mutex> g(err_mu_); err_ = msg; return code; }
   std::mutex err_mu_;
   std::vector<mvr_ctx*> ctx_;
@@ -177,5 +185,8 @@ int refineAxisFromPoses(const std::vector<Matrix4d>& poses, double pivot[3], dou
 // the source normals of ctxs[k], kept as that cloud's normals; a context may appear once per cloud.  which = NULL: all targets.
 int estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int count, int k, const float* viewpoints, float* const* out_nxyzc,
                            int* statuses);
+// mvr_score_guesses_batch with scored[k] (nullable) = the source points context k scored (api.cu; not part of the C ABI).
+int score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
+                        uint64_t* costs, int32_t* inliers, int* statuses, int32_t* scored);
 
 }  // namespace mvr

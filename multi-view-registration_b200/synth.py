@@ -101,11 +101,12 @@ def view_pose(view, n_views):
     return np.linalg.inv(rotation_about_axis(view * 2.0 * np.pi / n_views))
 
 
-def turntable_view(view, n_views, n, noise=0.2, seed=0x5EED0000, partial=True):
+def turntable_view(view, n_views, n, noise=0.2, seed=0x5EED0000, partial=True, angles=None):
     """Scan `view` of an n_views turntable sequence: (points n x 4 float32 in the sensor frame,
-    ground-truth pose 4x4 double mapping them into the frame of view 0)."""
+    ground-truth pose 4x4 double mapping them into the frame of view 0).  angles (optional, indexed by view): the table's
+    actual turn for each view instead of the ideal view * 2 pi / n_views (a table that steps unevenly)."""
     s = seed + view
-    theta = view * 2.0 * np.pi / n_views           # the table has turned the object by +theta
+    theta = view * 2.0 * np.pi / n_views if angles is None else float(angles[view])   # the table has turned the object by +theta
     R = rotation_about_axis(theta)
     kept = []
     have = 0
@@ -129,6 +130,18 @@ def turntable_view(view, n_views, n, noise=0.2, seed=0x5EED0000, partial=True):
     return _xyzw(p), np.linalg.inv(R)
 
 
+def step_errors(n_views, max_deg, seed=0x5EED0000):
+    """Seeded per-view turn errors (radians), uniform in [-max_deg, +max_deg] degrees; view 0 has none (it defines the frame)."""
+    e = np.deg2rad(max_deg) * (2.0 * uniform(seed ^ 0x57E9, np.arange(n_views, dtype=np.uint64)) - 1.0)
+    e[0] = 0.0
+    return e
+
+
+def uneven_angles(n_views, max_deg, seed=0x5EED0000):
+    """Turns of a table that steps unevenly: view * 2 pi / n_views + step_errors(...)[view]."""
+    return np.arange(n_views) * (2.0 * np.pi / n_views) + step_errors(n_views, max_deg, seed)
+
+
 def perturbation(seed=0x5EED0000, angle_deg=2.0, trans_mm=2.0):
     """Fixed small rigid error put on every initial guess: rotation about a seeded axis through the
     object centre plus a seeded translation."""
@@ -138,11 +151,11 @@ def perturbation(seed=0x5EED0000, angle_deg=2.0, trans_mm=2.0):
     return E
 
 
-def turntable_sequence(n_views, n, noise=0.2, seed=0x5EED0000):
-    """views (list of n x 4 float32), gt poses (list of 4x4 double, view -> frame of view 0)."""
+def turntable_sequence(n_views, n, noise=0.2, seed=0x5EED0000, angles=None):
+    """views (list of n x 4 float32), gt poses (list of 4x4 double, view -> frame of view 0); angles: see turntable_view."""
     views, poses = [], []
     for v in range(n_views):
-        p, T = turntable_view(v, n_views, n, noise=noise, seed=seed)
+        p, T = turntable_view(v, n_views, n, noise=noise, seed=seed, angles=angles)
         views.append(p)
         poses.append(T)
     return views, poses
