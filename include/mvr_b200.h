@@ -267,6 +267,52 @@ int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const flo
 int mvr_score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
                             uint64_t* costs, int32_t* inliers, int* statuses);
 
+/* -- global registration without an initial guess (pcl::FPFHEstimation + pcl::SampleConsensusPrerejective) ------------ */
+/* FPFH descriptors of a cloud's keypoints: the finite points of original index i % stride == 0, stride = max(1, ceil(n /
+ * keypoints)), in index order (at most `keypoints` of them).  Their kNN(k) PCA normals and neighbour lists are those
+ * mvr_estimate_normals gives for the keypoints set as a cloud of their own (same bits), flipped towards viewpoint (NULL: the
+ * centre of the cloud's bounding box, (lo + hi) * 0.5f); they do not replace the cloud's normals.  Per keypoint, over the first
+ * k - 1 entries of its list that are not itself: PCL's pair features in double, 11 bins each, every pair adding 100 / (k - 1)
+ * (SPFH); then FPFH = SPFH + the neighbours' SPFH weighted by 1 / d2, each sub-histogram of that sum scaled to 100, narrowed
+ * to float.  A keypoint whose normal is not finite gets an all-zero descriptor (it never matches).  index: keypoints int32
+ * (original indices), nxyzc (nullable): keypoints x 4, features: keypoints x 33; *n_kp = the keypoints found.
+ * keypoints: 1..65536, k: 8..32.  MVR_ERR_NO_INPUT if the cloud is not set; an empty cloud gives *n_kp = 0. */
+int mvr_compute_fpfh(mvr_ctx* ctx, int which /* mvr_cloud */, int keypoints, int k, const float viewpoint[3], int32_t* index, float* nxyzc,
+                     float* features, int* n_kp);
+/* Exact nearest descriptor (33 floats per row, host arrays) both ways: a_to_b[i] = the row of b nearest to row i of a in squared
+ * L2 summed over bins 0..32 in order without FMA, ties to the lowest row; b_to_a likewise.  All-zero rows never match (-1). */
+int mvr_match_features(mvr_ctx* ctx, const float* a, int na, const float* b, int nb, int32_t* a_to_b, int32_t* b_to_a);
+typedef struct {
+  int keypoints;        /* per cloud, 1..65536 (4096) */
+  int k;                /* neighbours of the normals and features, 8..32 (32) */
+  double max_dist;      /* gate of the hypothesis score, > 0 (4) */
+  int hypotheses;       /* accepted hypotheses to score, >= 1 (2048) */
+  int max_draws;        /* draws before giving up, >= 1 (1000000) */
+  double similarity;    /* edge-length similarity of a draw, 0..1 (0.9) */
+  double min_edge;      /* shortest source edge of a draw, as a fraction of the source keypoints' bbox diagonal (0.05) */
+  int samples;          /* source points per score, 1..65536 (4096) */
+  uint64_t seed;        /* of the draws' splitmix64 stream (0) */
+} mvr_global_params;
+typedef struct {
+  int matches;          /* mutual feature matches */
+  int draws;            /* triples drawn */
+  int hypotheses;       /* triples accepted and scored */
+  int best;             /* index of the best hypothesis (-1: none) */
+  uint64_t cost;        /* its mvr_score_guesses_batch cost */
+  int inliers;          /* its samples within max_dist */
+  int samples;          /* the source samples scored */
+  double gpu_ms;        /* device time of the features, the matching and the scoring (CUDA events on the context's stream) */
+} mvr_global_report;
+void mvr_global_params_default(mvr_global_params* p);
+/* The rigid pose (float[16] column-major) that maps the context's source onto its target, with no initial guess: FPFH of both
+ * clouds, mutual matches, triples of matches drawn from a splitmix64 stream of `seed` (a draw is rejected when a source edge is
+ * shorter than min_edge or an edge-length ratio is below similarity), each accepted triple fitted rigidly (Umeyama, double,
+ * narrowed to float), every hypothesis scored by mvr_score_guesses_batch(max_dist, samples); the lowest cost wins (ties: the
+ * lower index).  A pure function of the two clouds and the parameters.  Fewer than 3 mutual matches or no accepted draw:
+ * MVR_ERR_TOO_FEW_CORRESPONDENCES with out_pose = identity.  Refine with mvr_icp_align from out_pose: the context serves it
+ * as before (an align with the same max_dist reuses the scorer's target index). */
+int mvr_global_align(mvr_ctx* ctx, const mvr_global_params* params, float* out_pose, mvr_global_report* report);
+
 /* -- pose application: PointCloud::getTransformedPoints (mvr/src/point_cloud.cpp:290-303) ------------
  * out[i] = {float(pose * p_i), 1}: the multiply runs in double (osg::Matrix is double) and is narrowed to
  * float, RGB / normal lanes are dropped.  in: n records of `stride_bytes` bytes whose first three floats

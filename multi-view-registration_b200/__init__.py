@@ -125,6 +125,22 @@ class AnglePick(C.Structure):
                     guess_cost=int(self.guess_cost), guess_inliers=self.guess_inliers)
 
 
+class GlobalParams(C.Structure):
+    """mvr_global_params: the settings of Context.global_align (mvr_global_params_default: PCL-style defaults)."""
+    _fields_ = [("keypoints", C.c_int), ("k", C.c_int), ("max_dist", C.c_double), ("hypotheses", C.c_int), ("max_draws", C.c_int),
+                ("similarity", C.c_double), ("min_edge", C.c_double), ("samples", C.c_int), ("seed", C.c_uint64)]
+
+
+class GlobalReport(C.Structure):
+    """mvr_global_report: what Context.global_align found (best = index of the winning hypothesis, -1: none)."""
+    _fields_ = [("matches", C.c_int), ("draws", C.c_int), ("hypotheses", C.c_int), ("best", C.c_int), ("cost", C.c_uint64),
+                ("inliers", C.c_int), ("samples", C.c_int), ("gpu_ms", C.c_double)]
+
+    def as_dict(self):
+        return dict(matches=self.matches, draws=self.draws, hypotheses=self.hypotheses, best=self.best, cost=int(self.cost),
+                    inliers=self.inliers, samples=self.samples, gpu_ms=self.gpu_ms)
+
+
 class ViewDesc(C.Structure):
     _fields_ = [("xyzw", C.c_void_p), ("n", C.c_size_t), ("on_device", C.c_int), ("init_pose", C.POINTER(C.c_double))]
 
@@ -222,6 +238,11 @@ def lib():
     L.mvr_estimate_normals_batch.argtypes = [C.POINTER(vp), C.c_int, C.c_int, fp, C.POINTER(fp), ip]
     dp = C.POINTER(C.c_double)
     L.mvr_score_guesses_batch.argtypes = [C.POINTER(vp), C.c_int, fp, C.c_int, C.c_double, C.c_int, C.POINTER(C.c_uint64), ip, ip]
+    L.mvr_compute_fpfh.argtypes = [vp, C.c_int, C.c_int, C.c_int, fp, ip, fp, fp, C.POINTER(C.c_int)]
+    L.mvr_match_features.argtypes = [vp, fp, C.c_int, fp, C.c_int, ip, ip]
+    L.mvr_global_params_default.argtypes = [C.POINTER(GlobalParams)]
+    L.mvr_global_params_default.restype = None
+    L.mvr_global_align.argtypes = [vp, C.POINTER(GlobalParams), fp, C.POINTER(GlobalReport)]
     L.mvr_angle_search_default.argtypes = [C.POINTER(AngleSearch)]
     L.mvr_angle_search_default.restype = None
     L.mvr_registrator_set_angle_search.argtypes = [vp, C.POINTER(AngleSearch)]
@@ -552,6 +573,40 @@ class Context:
         return (out, nbr) if want_neighbours else out
 
 
+    def fpfh(self, which, keypoints, k, viewpoint=None):
+        """mvr_compute_fpfh: (original indices of the keypoints int32, their normals n_kp x 4, FPFH n_kp x 33 float32).
+        viewpoint None: the centre of the cloud's bounding box."""
+        vp = None if viewpoint is None else np.ascontiguousarray(viewpoint, dtype=np.float32)
+        idx = np.empty(int(keypoints), dtype=np.int32)
+        nrm = np.empty((int(keypoints), 4), dtype=np.float32)
+        feat = np.empty((int(keypoints), 33), dtype=np.float32)
+        n = C.c_int(0)
+        self._ck(lib().mvr_compute_fpfh(self._h, int(which), int(keypoints), int(k), _fp(vp) if vp is not None else None, _ip(idx), _fp(nrm),
+                                        _fp(feat), C.byref(n)))
+        m = n.value
+        return idx[:m].copy(), nrm[:m].copy(), feat[:m].copy()
+
+    def match_features(self, a, b):
+        """mvr_match_features: (a_to_b, b_to_a) exact nearest rows of two n x 33 float32 descriptor tables (-1: none)."""
+        a = np.ascontiguousarray(a, dtype=np.float32).reshape(-1, 33)
+        b = np.ascontiguousarray(b, dtype=np.float32).reshape(-1, 33)
+        ab = np.empty(max(len(a), 1), dtype=np.int32)
+        ba = np.empty(max(len(b), 1), dtype=np.int32)
+        self._ck(lib().mvr_match_features(self._h, _fp(a), len(a), _fp(b), len(b), _ip(ab), _ip(ba)))
+        return ab[:len(a)].copy(), ba[:len(b)].copy()
+
+    def global_align(self, params=None):
+        """mvr_global_align: (pose 4x4 float32 mapping the source onto the target, report dict with status).  A status of
+        MVR_ERR_TOO_FEW_CORRESPONDENCES is reported (pose = identity), not raised."""
+        p = params if params is not None else global_params()
+        out = np.empty(16, dtype=np.float32)
+        rep = GlobalReport()
+        rc = lib().mvr_global_align(self._h, C.byref(p), _fp(out), C.byref(rep))
+        self._ck(rc, allow=(ERR_TOO_FEW,))
+        d = rep.as_dict()
+        d["status"] = rc
+        return pose_to_numpy(out), d
+
     def denoise(self, pts, segment_threshold=10, triangle_length=2.5):
         """PointCloud::denoise: (indices of the kept points in the reference's output order, number of noise points).
         pts: n x 4 float32 (PointXYZ) or a RICH_POINT array (48-byte records)."""
@@ -754,6 +809,15 @@ def score_guesses_batch(contexts, candidates, max_dist, samples=4096):
     if rc != OK:
         raise MvrError(rc, contexts[0].last_error() if n else lib().mvr_status_string(rc).decode())
     return costs[:n], inl[:n], st[:n]
+
+
+def global_params(**kw):
+    """mvr_global_params with the library's defaults, overridden by keyword."""
+    p = GlobalParams()
+    lib().mvr_global_params_default(C.byref(p))
+    for k, v in kw.items():
+        setattr(p, k, v)
+    return p
 
 
 def angle_search_default():

@@ -13,8 +13,8 @@ CSRC = os.path.join(HERE, "csrc")
 HOST = os.path.join(HERE, "host")
 LIB = os.path.join(HERE, "libmvr_b200.so")
 
-CU_SOURCES = ["index.cu", "pair_index.cu", "cell_nn.cu", "icp.cu", "normals.cu", "denoise.cu", "score.cu", "api.cu"]
-HOST_SOURCES = ["registrator.cpp", "lum.cpp", "capi.cpp", "multi.cpp"]
+CU_SOURCES = ["index.cu", "pair_index.cu", "cell_nn.cu", "icp.cu", "normals.cu", "denoise.cu", "score.cu", "features.cu", "api.cu"]
+HOST_SOURCES = ["registrator.cpp", "lum.cpp", "capi.cpp", "multi.cpp", "global.cpp"]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17",

@@ -36,6 +36,8 @@ int estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int count, in
                            int* statuses);
 int score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
                         uint64_t* costs, int32_t* inliers, int* statuses, int32_t* scored);
+int compute_fpfh(mvr_ctx* ctx, int which, int keypoints, int k, const float* viewpoint, int32_t* index, float* nxyzc, float* features,
+                 int* n_kp, float* kp_xyzw);
 }  // namespace mvr
 
 namespace {
@@ -131,6 +133,9 @@ struct mvr_ctx {
   DevBuf score_dev;              // mvr_score_guesses_batch led by this context: candidate table, then the sums
   unsigned char* h_score = nullptr;   // pinned staging of the same layout, score_cap bytes
   size_t score_cap = 0;
+  // mvr_compute_fpfh / mvr_match_features: keypoints, their indices, normals, neighbour lists, SPFH scratch, descriptors; the
+  // matcher's two descriptor tables and its results
+  DevBuf kp, kp_idx, kp_nrm, kp_nbr, kp_spfh, kp_feat, mt_a, mt_b, mt_out;
   int log_pending = 0;           // records of the device log not fetched yet (mvr_icp_get_iterations fetches them)
   bool out_pending = false;      // out_cloud has not been computed yet (materialize_out)
   DevBuf crowded;                        // one word: population of the most crowded cell an index build could not rank (0: none)
@@ -643,6 +648,7 @@ int mvr_ctx_destroy(mvr_ctx* ctx) {
   ctx->pt.release(); ctx->ps.release(); ctx->nt.release(); ctx->nq.release();
   for (auto& b : ctx->bs) { b.keys.release(); b.vals.release(); b.moved.release(); b.count.release(); b.tiles.release(); }
   ctx->stage_dev.release(); ctx->bbox_dev.release(); ctx->score_dev.release();
+  for (DevBuf* b : {&ctx->kp, &ctx->kp_idx, &ctx->kp_nrm, &ctx->kp_nbr, &ctx->kp_spfh, &ctx->kp_feat, &ctx->mt_a, &ctx->mt_b, &ctx->mt_out}) b->release();
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_bbox) cudaFreeHost(ctx->h_bbox);
   if (ctx->h_score) cudaFreeHost(ctx->h_score);
@@ -1903,6 +1909,99 @@ int mvr_estimate_normals_batch(mvr_ctx* const* ctxs, int count, int k, const flo
 int mvr_score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
                             uint64_t* costs, int32_t* inliers, int* statuses) {
   return mvr::score_guesses_batch(ctxs, count, candidates, n_candidates, max_dist, samples, costs, inliers, statuses, nullptr);
+}
+
+}  // extern "C"
+
+// ---- features of the global registration (features.cu, host/global.cpp) ------------------------------------------------
+// The keypoints are gathered into a compact buffer of their own and given the index, grid and kernel mvr_estimate_normals would
+// give them as a cloud (the same bits): their bounding box is measured by the same launch, the index lives in the query index
+// (nq, invalidated afterwards, as mvr_estimate_normals leaves it).  The cloud's own normals (tnrm / snrm) are untouched.
+int mvr::compute_fpfh(mvr_ctx* ctx, int which, int keypoints, int k, const float* viewpoint, int32_t* index, float* nxyzc, float* features,
+                      int* n_kp, float* kp_xyzw) {
+  if (!ctx || !index || !features || !n_kp || (which != MVR_CLOUD_TARGET && which != MVR_CLOUD_SOURCE)) return MVR_ERR_BAD_ARG;
+  if (keypoints < 1 || keypoints > 65536) return fail(ctx, MVR_ERR_BAD_ARG, "keypoints must be in 1..65536");
+  if (k < 8 || k > 32) return fail(ctx, MVR_ERR_BAD_ARG, "k must be in 8..32");
+  *n_kp = 0;
+  cudaSetDevice(ctx->device);
+  const Cloud& c = which == MVR_CLOUD_TARGET ? ctx->tgt : ctx->src;
+  if (c.gen == 0) return fail(ctx, MVR_ERR_NO_INPUT, "cloud not set");
+  const int n = c.n;
+  if (n - c.n_bad <= 0) return MVR_OK;
+  const int stride = std::max(1, (int)(((long long)n + keypoints - 1) / keypoints));
+  const int slots = (n + stride - 1) / stride;
+  const cudaStream_t S = ctx->stream;
+  CK(ctx->kp.ensure((size_t)slots * sizeof(float4)));
+  CK(ctx->kp_idx.ensure((size_t)slots * sizeof(int32_t)));
+  CK(ctx->kp_nrm.ensure((size_t)slots * sizeof(float4)));
+  CK(ctx->kp_nbr.ensure((size_t)slots * k * sizeof(int32_t)));
+  CK(ctx->kp_spfh.ensure((size_t)slots * 33 * sizeof(double)));
+  CK(ctx->kp_feat.ensure((size_t)slots * 33 * sizeof(float)));
+  CK(ctx->misc.ensure(64));
+  float4* kp = ctx->kp.as<float4>();
+  {
+    ProfScope ps(ctx, MVR_K_NORMALS, 16.0 * slots + 24.0 * slots, slots);
+    CK(launch_keypoints(c.pts, stride, slots, kp, ctx->kp_idx.as<int32_t>(), S));
+    CK(launch_bbox_init(ctx->misc.as<uint32_t>(), S));
+    CK(launch_bbox(kp, slots, ctx->misc.as<uint32_t>(), S));
+  }
+  CK(cudaMemcpyAsync(ctx->h_small, ctx->misc.p, 7 * sizeof(uint32_t), cudaMemcpyDeviceToHost, S));
+  CK(cudaStreamSynchronize(S));
+  Cloud kc;   // the keypoints as a cloud: what the grid choice reads
+  kc.n = slots - (int)ctx->h_small[6];
+  for (int a = 0; a < 3; ++a) { kc.lo[a] = bbox_decode(ctx->h_small[a]); kc.hi[a] = bbox_decode(ctx->h_small[3 + a]); }
+  const int m = kc.n;
+  float vp[3];
+  for (int a = 0; a < 3; ++a) vp[a] = viewpoint ? viewpoint[a] : (c.lo[a] + c.hi[a]) * 0.5f;
+  uint32_t cells = 0;
+  const PairGrid g = normals_grid(ctx, kc, k, &cells);
+  PairIndex& ix = ctx->nq;
+  int rc = build_pair_index(ctx, ix, kp, m, 0, nullptr, g, cells, false);
+  if (rc) return rc;
+  NormalsBatch batch;
+  batch.j[0] = normals_job(ix, m, vp, ctx->kp_nrm.as<float4>(), ctx->kp_nbr.as<int32_t>());
+  {
+    ProfScope ps(ctx, MVR_K_NORMALS, 32.0 * m + (double)m * k * 4.0 + (double)m * 33.0 * (8.0 + 8.0 + 4.0) + (double)m * (k - 1) * (32.0 + 33.0 * 8.0), m);
+    CK(launch_normals(batch, 1, k, S));
+    CK(launch_fpfh(kp, ctx->kp_nrm.as<float4>(), ctx->kp_nbr.as<int32_t>(), m, k, ctx->kp_spfh.as<double>(), ctx->kp_feat.as<float>(), S));
+  }
+  ix.valid = false;
+  CK(cudaMemcpyAsync(index, ctx->kp_idx.p, (size_t)m * sizeof(int32_t), cudaMemcpyDeviceToHost, S));
+  CK(cudaMemcpyAsync(features, ctx->kp_feat.p, (size_t)m * 33 * sizeof(float), cudaMemcpyDeviceToHost, S));
+  if (nxyzc) CK(cudaMemcpyAsync(nxyzc, ctx->kp_nrm.p, (size_t)m * sizeof(float4), cudaMemcpyDeviceToHost, S));
+  if (kp_xyzw) CK(cudaMemcpyAsync(kp_xyzw, kp, (size_t)m * sizeof(float4), cudaMemcpyDeviceToHost, S));
+  CK(cudaStreamSynchronize(S));
+  *n_kp = m;
+  return MVR_OK;
+}
+
+extern "C" {
+
+int mvr_compute_fpfh(mvr_ctx* ctx, int which, int keypoints, int k, const float viewpoint[3], int32_t* index, float* nxyzc, float* features,
+                     int* n_kp) {
+  return mvr::compute_fpfh(ctx, which, keypoints, k, viewpoint, index, nxyzc, features, n_kp, nullptr);
+}
+
+int mvr_match_features(mvr_ctx* ctx, const float* a, int na, const float* b, int nb, int32_t* a_to_b, int32_t* b_to_a) {
+  if (!ctx || na < 0 || nb < 0 || (na && (!a || !a_to_b)) || (nb && (!b || !b_to_a))) return MVR_ERR_BAD_ARG;
+  cudaSetDevice(ctx->device);
+  const cudaStream_t S = ctx->stream;
+  const size_t ba = (size_t)na * 33 * sizeof(float), bb = (size_t)nb * 33 * sizeof(float);
+  CK(ctx->mt_a.ensure(std::max<size_t>(ba, 4)));
+  CK(ctx->mt_b.ensure(std::max<size_t>(bb, 4)));
+  CK(ctx->mt_out.ensure(((size_t)na + nb + 1) * sizeof(int32_t)));
+  if (na) CK(cudaMemcpyAsync(ctx->mt_a.p, a, ba, cudaMemcpyHostToDevice, S));
+  if (nb) CK(cudaMemcpyAsync(ctx->mt_b.p, b, bb, cudaMemcpyHostToDevice, S));
+  int32_t* out = ctx->mt_out.as<int32_t>();
+  {
+    ProfScope ps(ctx, MVR_K_NN, 2.0 * (double)na * nb * 33.0 * 4.0 / 128.0 + (double)(ba + bb), (double)na + nb);
+    CK(launch_match(ctx->mt_a.as<float>(), na, ctx->mt_b.as<float>(), nb, out, S));
+    CK(launch_match(ctx->mt_b.as<float>(), nb, ctx->mt_a.as<float>(), na, out + na, S));
+  }
+  if (na) CK(cudaMemcpyAsync(a_to_b, out, (size_t)na * sizeof(int32_t), cudaMemcpyDeviceToHost, S));
+  if (nb) CK(cudaMemcpyAsync(b_to_a, out + na, (size_t)nb * sizeof(int32_t), cudaMemcpyDeviceToHost, S));
+  CK(cudaStreamSynchronize(S));
+  return MVR_OK;
 }
 
 }  // extern "C"

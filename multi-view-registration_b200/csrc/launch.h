@@ -276,4 +276,14 @@ static_assert(sizeof(ScoreBatch) + sizeof(int) <= 32764, "the batch's jobs must 
 // `count` (<= BUILD_MAX_JOBS) contexts, all with nc (<= SCORE_MAX_CANDIDATES) candidates, in one launch (blockIdx.y = context).
 cudaError_t launch_score(const ScoreBatch& batch, int count, int nc, cudaStream_t s);
 
+// ---- features.cu --------------------------------------------------------------------------------
+// The keypoints of a cloud: the finite points of original index s * stride (s < slots) in index order go to out[0 .. n_kp) with
+// index[] = their original index; out[n_kp .. slots) = NaN, index = -1.  One block.
+cudaError_t launch_keypoints(const float4* pts, int stride, int slots, float4* out, int32_t* index, cudaStream_t s);
+// FPFH (33 floats per keypoint) of n keypoints from their normals and k_normals neighbour lists (n x k, keypoint indices);
+// spfh: scratch, n x 33 doubles.  Two launches.
+cudaError_t launch_fpfh(const float4* kp, const float4* nrm, const int32_t* nbr, int n, int k, double* spfh, float* out, cudaStream_t s);
+// out[i] = nearest row of b (nb x 33) to row i of a (na x 33), exact; -1: none (all-zero rows never match).
+cudaError_t launch_match(const float* a, int na, const float* b, int nb, int32_t* out, cudaStream_t s);
+
 }  // namespace mvr

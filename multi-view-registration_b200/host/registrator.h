@@ -188,5 +188,8 @@ int estimate_normals_batch(mvr_ctx* const* ctxs, const int* which, int count, in
 // mvr_score_guesses_batch with scored[k] (nullable) = the source points context k scored (api.cu; not part of the C ABI).
 int score_guesses_batch(mvr_ctx* const* ctxs, int count, const float* candidates, int n_candidates, double max_dist, int samples,
                         uint64_t* costs, int32_t* inliers, int* statuses, int32_t* scored);
+// mvr_compute_fpfh with kp_xyzw (nullable, keypoints x 4) = the keypoints' points (api.cu; not part of the C ABI).
+int compute_fpfh(mvr_ctx* ctx, int which, int keypoints, int k, const float* viewpoint, int32_t* index, float* nxyzc, float* features,
+                 int* n_kp, float* kp_xyzw);
 
 }  // namespace mvr

@@ -101,13 +101,32 @@ def view_pose(view, n_views):
     return np.linalg.inv(rotation_about_axis(view * 2.0 * np.pi / n_views))
 
 
-def turntable_view(view, n_views, n, noise=0.2, seed=0x5EED0000, partial=True, angles=None):
+def random_placement(seed):
+    """A seeded arbitrary rigid move of the object about CENTER (4x4 double): a uniform random rotation (unit quaternion of
+    four seeded normals) and a translation up to +-200 mm per axis -- the object put back on the table in another pose."""
+    g = _gauss3(seed ^ 0x91ACE, np.arange(2, dtype=np.uint64)).reshape(-1)[:4]
+    w, x, y, z = g / np.linalg.norm(g)
+    Rq = np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y)],
+                   [2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x)],
+                   [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
+    t = 400.0 * uniform(seed ^ 0x7A55, np.arange(3, dtype=np.uint64)) - 200.0
+    M = np.eye(4)
+    M[:3, :3] = Rq
+    M[:3, 3] = CENTER - Rq @ CENTER + t
+    return M
+
+
+def turntable_view(view, n_views, n, noise=0.2, seed=0x5EED0000, partial=True, angles=None, placement=None):
     """Scan `view` of an n_views turntable sequence: (points n x 4 float32 in the sensor frame,
     ground-truth pose 4x4 double mapping them into the frame of view 0).  angles (optional, indexed by view): the table's
-    actual turn for each view instead of the ideal view * 2 pi / n_views (a table that steps unevenly)."""
+    actual turn for each view instead of the ideal view * 2 pi / n_views (a table that steps unevenly).  placement (optional
+    4x4 rigid move): the object is moved by it before the table turns (placed on its side, upside down, ...); the pose still
+    maps the view into the frame of view 0 of the same placement."""
     s = seed + view
     theta = view * 2.0 * np.pi / n_views if angles is None else float(angles[view])   # the table has turned the object by +theta
     R = rotation_about_axis(theta)
+    if placement is not None:
+        R = R @ np.asarray(placement, dtype=np.float64)
     kept = []
     have = 0
     start = 0
@@ -127,6 +146,8 @@ def turntable_view(view, n_views, n, noise=0.2, seed=0x5EED0000, partial=True, a
         kept.append(p)
         have += len(p)
     p = np.concatenate(kept)[:n]
+    if placement is not None:
+        return _xyzw(p), np.linalg.inv(rotation_about_axis(theta))
     return _xyzw(p), np.linalg.inv(R)
 
 
@@ -151,11 +172,12 @@ def perturbation(seed=0x5EED0000, angle_deg=2.0, trans_mm=2.0):
     return E
 
 
-def turntable_sequence(n_views, n, noise=0.2, seed=0x5EED0000, angles=None):
-    """views (list of n x 4 float32), gt poses (list of 4x4 double, view -> frame of view 0); angles: see turntable_view."""
+def turntable_sequence(n_views, n, noise=0.2, seed=0x5EED0000, angles=None, placement=None):
+    """views (list of n x 4 float32), gt poses (list of 4x4 double, view -> frame of view 0); angles, placement: see
+    turntable_view."""
     views, poses = [], []
     for v in range(n_views):
-        p, T = turntable_view(v, n_views, n, noise=noise, seed=seed, angles=angles)
+        p, T = turntable_view(v, n_views, n, noise=noise, seed=seed, angles=angles, placement=placement)
         views.append(p)
         poses.append(T)
     return views, poses
